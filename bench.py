@@ -2,7 +2,7 @@
 """bench.py - dBG build throughput (G k-mers/s) of the B200 path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload cfg2|cfg3|cfg4|cfg5|small|cfg4s] [--k 27]
+                    [--workload cfg2|cfg3|cfg4|cfg5|small|cfg4s] [--k 27] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A *step* is one full dBG build of the workload: FASTA scan/pack (K1) + table reset +
 k-mer extraction into hash-partitioned compact 8-byte update records (K2a-c; across GPUs fused with the exchange over
@@ -21,6 +21,9 @@ upserts.  Metric = k-mer insertions / s, an insertion being one k-mer occurrence
            (oracle/, kind "port"), one core, on a bounded sample of the same workload.
  checksum: the built table's order-independent checksum, compared with the oracle's (configs 2 / 3) or the recorded one
            (configs 4 / 5) BEFORE anything is timed: a line is only printed for a correct table.
+
+--dump-outputs DIR writes the table the last timed step built as DIR/<name>.npy (see dump_outputs), so that two builds
+of the project can be compared output for output on the same seeded workload.
 """
 import argparse
 import json
@@ -219,6 +222,35 @@ def golden_checksum(workload_name, k, scale):
         return None, None
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, table, world=1, rank=0, seed=0):
+    """Write ``table`` (what RoundBuilder.build_async returned) as float arrays under ``out_dir``: its exported entries in
+    key order - the 64-bit base-5 key split into exact 32-bit halves (float64 holds 53 bits), value and count - with
+    their positions in that order, and the table's (entries, sum, xor) checksum, 64-bit words split the same way.  A
+    table with more entries than DUMP_BYTES allows is written as a fixed, seeded sample of positions.  With several
+    ranks every rank writes its own part (``_rank<r>`` names) within its share of DUMP_BYTES."""
+    import numpy as np
+    ks, vs, cs = table.export()
+    n, s, x = table.checksum()
+    per_entry = 8 + 8 + 4 + 4 + 8                       # key_hi, key_lo, position (float64), value, count (float32)
+    cap = (DUMP_BYTES // world - 4096) // per_entry
+    pos = np.arange(ks.size) if ks.size <= cap else np.sort(np.random.default_rng(seed).choice(ks.size, cap, replace=False))
+    arrays = {
+        "dbg_key_hi": (ks[pos] >> np.uint64(32)).astype(np.float64),
+        "dbg_key_lo": (ks[pos] & np.uint64(0xFFFFFFFF)).astype(np.float64),
+        "dbg_value": vs[pos].astype(np.float32),
+        "dbg_count": cs[pos].astype(np.float32),
+        "dbg_position": pos.astype(np.float64),
+        "dbg_checksum": np.array([n, s >> 32, s & 0xFFFFFFFF, x >> 32, x & 0xFFFFFFFF], dtype=np.float64),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -231,6 +263,9 @@ def main():
     ap.add_argument("--rounds", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-stages", action="store_true", help="skip the K1/K4..K8 roofline entries and the atomic ceiling")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the table the last timed step built as DIR/<name>.npy (float32 / float64, <= 64 MB; --impl ours). "
+                         "Untimed, but it exports the whole table: 11 B of device memory per entry and a host sort")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.workload is None:
@@ -239,6 +274,10 @@ def main():
     big = WORKLOADS.get(args.workload, ("", "", 0, 0))[2] * WORKLOADS.get(args.workload, ("", "", 0, 0))[3] * args.scale > 5e8
     if args.steps is None:
         args.steps = 10 if big else 50
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU build's table: it needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference_arm(args)
@@ -331,6 +370,8 @@ def main():
     torch.cuda.synchronize()
     clk = clocks.stop() if clocks else None
     bld.verify()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, t, world, rank)     # before the steps below rebuild into the same table
     ms_step = allmax(e0.elapsed_time(e1)) / args.steps
     value = n_ins / (ms_step * 1e-3) / 1e9
     # per-stage times (the roofline entries): the same steps again with CUDA events around every kernel group, outside the

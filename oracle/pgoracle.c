@@ -79,6 +79,12 @@ static uint64_t fnv4(uint64_t val) {        /* :400-411, ksize==1 branch: low 4 
     for (int i = 0; i < 4; i++) { a ^= (val & 0xff); a *= 0x100000001b3ull; val >>= 8; }
     return a;
 }
+/* first probe slot: the reference hashes in int64 and numba's % is Python's floor modulo, so a hash with bit 63 set
+   starts at (signed hash) mod M, not at the unsigned remainder */
+static int64_t oakht_slot0(uint64_t key, int64_t M) {
+    int64_t j = (int64_t)fnv4(key) % M;
+    return j < 0 ? j + M : j;
+}
 static void oakht_init(oakht *h) {          /* :341-352; init_dict ignores `capacity` (:1121) */
     h->capacity = find_prime(1 << 20);
     h->load = 0.75f; h->size = 0; h->n_probe = 0;
@@ -90,7 +96,7 @@ static void oakht_free(oakht *h) { free(h->keys); free(h->values); free(h->count
 
 static int64_t oakht_pointer(oakht *h, uint64_t key) {   /* :521-538 */
     int64_t M = h->capacity;
-    int64_t j = (int64_t)(fnv4(key) % (uint64_t)M), j_init = j;
+    int64_t j = oakht_slot0(key, M), j_init = j;
     for (int64_t k = 0; k < M; k++) {
         if (h->keys[j] == key || h->counts[j] == 0) break;   /* equality tested BEFORE occupancy: Q6 */
         j = (j_init + k * k) % M;
@@ -103,7 +109,7 @@ static void oakht_resize(oakht *h) {        /* :423-474 */
     uint64_t *keys = calloc((size_t)M, 8); uint16_t *values = calloc((size_t)M, 2); uint8_t *counts = calloc((size_t)M, 1);
     for (int64_t i = 0; i < N; i++) {
         if (h->counts[i] == 0) continue;
-        int64_t j = (int64_t)(fnv4(h->keys[i]) % (uint64_t)M), j_init = j;
+        int64_t j = oakht_slot0(h->keys[i], M), j_init = j;
         for (int64_t k = 0; k < N; k++) {
             if (counts[j] == 0 || keys[j] == h->keys[i]) break;
             j = (j_init + k * k) % M;

@@ -63,7 +63,9 @@ extern "C" int pg_host_write_mcl(const char *path, const uint64_t *code, const u
 // The reference stores its dBG as the raw arrays of its open-addressing table `oakht`; to hand a
 // GPU-built dBG to the reference's `-d` option the entries must be laid out the way its `pointer()`
 // (:521-538) will probe for them: prime capacity, FNV-1a over the low 4 key bytes (:400-411),
-// quadratic probing j = (j0 + t*t) % M.  Host code: this is file-format work, not the hot path.
+// quadratic probing j = (j0 + t*t) % M.  The reference computes the hash in int64 and numba's % is
+// Python's floor modulo, so j0 = signed hash mod M in [0, M): for hashes with bit 63 set this is not
+// the unsigned remainder.  Host code: this is file-format work, not the hot path.
 namespace {
 bool oak_isprime(int64_t n) {
     if (n <= 1 || n % 2 == 0 || n % 3 == 0) return false;
@@ -91,7 +93,9 @@ extern "C" int pg_host_build_oakht(const uint64_t *keys, const uint16_t *vals, c
     if (n < 0 || cap < 1 || n > cap || !okeys || !ovals || !ocnts) return pg_fail(PG_ERR_INVALID, "pg_host_build_oakht: bad arguments");
     memset(okeys, 0, (size_t)cap * 8); memset(ovals, 0, (size_t)cap * 2); memset(ocnts, 0, (size_t)cap);
     for (int64_t i = 0; i < n; i++) {
-        int64_t j = (int64_t)(oak_fnv4(keys[i]) % (uint64_t)cap), j0 = j;
+        int64_t j = (int64_t)oak_fnv4(keys[i]) % cap;
+        if (j < 0) j += cap;
+        const int64_t j0 = j;
         for (int64_t t = 0; t < cap; t++) {
             if (ocnts[j] == 0 || okeys[j] == keys[i]) break;
             j = (j0 + t * t) % cap;

@@ -22,7 +22,10 @@ def emul():
     deps = [src] + [os.path.join(ROOT, "pangenome_b200", "csrc", f) for f in
                     ("fasta_chunk.cuh", "kmer_core.cuh", "common.cuh")]
     if not os.path.isfile(_SO) or any(os.path.getmtime(d) > os.path.getmtime(_SO) for d in deps):
-        subprocess.check_call(["nvcc", "-O2", "-std=c++17", "--shared", "-Xcompiler", "-fPIC", "-o", _SO, src])
+        # compiled under a private name and renamed into place: parallel test workers never load a half-written library
+        tmp = "%s.%d.so" % (_SO[:-3], os.getpid())
+        subprocess.check_call(["nvcc", "-O2", "-std=c++17", "--shared", "-Xcompiler", "-fPIC", "-o", tmp, src])
+        os.replace(tmp, _SO)
     L = ctypes.CDLL(_SO)
     L.emul_pack.restype = ctypes.c_int64
     L.emul_pack2.restype = ctypes.c_int64

@@ -1,17 +1,23 @@
 """`_db.npz` interop (SURVEY 8 f1).  CPU part: the oakht image written by pangenome_b200.npz is
-what the reference's own loader expects - checked by probing like `oakht.pointer` (always) and by
-running the reference's load_on_disk + dbg2rdbg on it (only where oracle/_ref exists).  GPU part:
+what the reference's own loader expects - checked by probing like `oakht.pointer`, against the
+images the reference itself wrote (its chunk checkpoints in tests/golden/chunk_cases.json), and by
+running the reference's load_on_disk + dbg2rdbg on it where oracle/_ref exists.  GPU part:
 `-d file.npz` produced by the reference-layout writer round-trips through the GPU table."""
+import base64
+import io
+import json
 import os
 
 import numpy as np
 import pytest
 
 import oracle
-from conftest import load_small_cases
+from conftest import GOLDEN, load_small_cases
 from oracle import refrun
 
 CASES = {c["name"]: c for c in load_small_cases()}
+with open(os.path.join(GOLDEN, "chunk_cases.json")) as f:
+    REF_IMAGES = [c for c in json.load(f) if c["brkpt_b64"] is not None]     # written by the reference's dump (:243-261)
 
 
 def _triples(case):
@@ -30,6 +36,12 @@ def _fnv4(v):
     return a
 
 
+def _slot0(key, M):
+    """First probe slot of oakht.pointer: the hash is an int64 there and numba's % is Python's floor modulo."""
+    h = _fnv4(key)
+    return (h - (1 << 64) if h >> 63 else h) % M
+
+
 @pytest.mark.parametrize("name", ["test_fsa_k5", "test_fsa_k27", "nasty_k11_lf", "rand05_k15_c2"])
 def test_oakht_image_is_probeable_like_the_reference(name):
     from pangenome_b200 import npz
@@ -41,7 +53,7 @@ def test_oakht_image_is_probeable_like_the_reference(name):
     assert params.tolist()[1:] == [750000000, keys.size, 1, 1, 0]
     M = int(params[0])
     for k_, v_, c_ in zip(keys.tolist(), vals.tolist(), cnts.tolist()):
-        j = _fnv4(k_) % M
+        j = _slot0(k_, M)
         j0, t = j, 0
         while not (int(ok[j]) == k_ or oc[j] == 0):      # oakht.pointer (:521-538)
             j = (j0 + t * t) % M
@@ -49,16 +61,34 @@ def test_oakht_image_is_probeable_like_the_reference(name):
         assert int(ok[j]) == k_ and ov[j] == v_ and oc[j] == c_
 
 
-@pytest.mark.skipif(not refrun.available(), reason="oracle/_ref (patched reference) not built on this machine")
 def test_reference_loads_our_image(tmp_path):
-    """The reference's load_on_disk + dbg2rdbg on an image we wrote -> the golden rdBG."""
+    """The image we write for a table is, slot for slot, the one the reference writes for it: compared with every
+    checkpoint image the reference wrote (and resumed from) in the golden chunk cases, so its load_on_disk reads back
+    its own layout and its pointer() finds every key.  The nasty_k11_lf image read back the way load_on_disk reads it
+    (live slots) is the reference's dBG, whose rdBG is the golden one; where oracle/_ref exists the reference's own
+    load_on_disk + dbg2rdbg run on that image as well."""
     from pangenome_b200 import npz
-    mod = refrun.load()
+    for ref in REF_IMAGES:
+        z = np.load(io.BytesIO(base64.b64decode(ref["brkpt_b64"])))
+        keys = np.array([e[0] for e in ref["brkpt_live"]], dtype=np.uint64)
+        vals = np.array([e[1] for e in ref["brkpt_live"]], dtype=np.uint16)
+        cnts = np.array([e[2] for e in ref["brkpt_live"]], dtype=np.uint8)
+        ours = npz.oakht_image(keys, vals, cnts, offset=ref["offset"])
+        for name, a in zip(("parameters", "keys", "values", "counts"), ours):
+            assert np.array_equal(a, z[name]), (ref["name"], name)
     case = CASES["nasty_k11_lf"]
     keys, vals, cnts = _triples(case)
     params, ok, ov, oc = npz.oakht_image(keys, vals, cnts)
     fn = str(tmp_path / "x_db")
     np.savez_compressed(fn, parameters=params, keys=ok, values=ov, counts=oc)
+    z = np.load(fn + ".npz")
+    live = z["counts"] > 0
+    assert int(z["parameters"][2]) == live.sum() == len(case["dbg"])
+    o = np.argsort(z["keys"][live], kind="stable")
+    assert [[int(a), int(b), int(c)] for a, b, c in zip(z["keys"][live][o], z["values"][live][o], z["counts"][live][o])] == case["dbg"]
+    if not refrun.available():
+        return
+    mod = refrun.load()
     offset, kd = mod.load_on_disk(fn + ".npz")
     assert kd.size == keys.size
     rd = mod.dbg2rdbg(kd)
