@@ -376,6 +376,64 @@ int pg_graph_export_edges(const pg_graph *g, const pg_table *rdbg, uint64_t *d_c
 int pg_graph_export_nodes(const pg_graph *g, const pg_table *rdbg, uint32_t *d_nslot, uint64_t *d_code, uint32_t *d_v5,
                           uint32_t *d_root, int64_t cap, int64_t *d_n, pg_stream_t stream);
 
+/* ---- K7m: Markov clustering of the rdBG edge graph (opt-in, `--cluster mcl`) -------------
+ * Replaces the external `mcl <xyz> --abc -I r` run (kmer_numba.py:1911).  The definition (DESIGN.md §3) is
+ * this project's: agreement with micans mcl is unverified.  Column-stochastic matrix M in CSC form
+ * (int64 column pointers, int32 rows ascending inside a column, float32 values); one iteration is
+ *   M <- normalise(inflate_r(prune(M.M)))
+ * with every float32 sum taken left to right (expansion: ascending k; column sums and sums of squares:
+ * ascending row) and correctly rounded operations only, so the CPU oracle matches bit for bit when r is a
+ * multiple of 1/2 (x^r = x^floor(r) by repeated products, times sqrt(x) for the half; any other r: powf).
+ * prune: keep the min(S, #entries >= theta) largest entries of a column (value descending, row ascending);
+ * a column with no entry >= theta keeps its largest one.  chaos_j = max_i M[i,j] / sum_i M[i,j]^2 - 1 after
+ * normalisation; the run stops when max_j chaos_j < tau or after T iterations.
+ *
+ * pg_mcl_normalise: normalise every column in place; d_stats[PG_MCL_STAT_CHAOS] = max_j max(chaos_j, 0)
+ *   (float bits), d_stats[PG_MCL_STAT_NNZ] = nonzeros.
+ * pg_mcl_plan: d_prod[j] = products of column j (sum of nnz(col k) over k in col j); d_stage_off = exclusive
+ *   scan of min(d_prod[j], S) (n + 1 entries: the staging size is d_stage_off[n]); columns with more than
+ *   PG_MCL_WARP_PRODUCTS products are listed in d_large (cap n) and counted in d_stats[PG_MCL_STAT_LARGE];
+ *   d_stats[PG_MCL_STAT_PRODUCTS] / [PG_MCL_STAT_MAXPROD] = total / largest product count.
+ * pg_mcl_expand: expansion + prune + inflation + normalisation of every column into the staging arrays
+ *   (column j at d_stage_off[j], d_kept[j] entries, rows ascending); columns up to PG_MCL_WARP_PRODUCTS
+ *   products take one warp each, larger ones one CTA each (shared-memory accumulator up to
+ *   PG_MCL_SMEM_SLOTS slots, else a slab of the caller's workspace d_ws per resident CTA; the slab holds
+ *   pg_mcl_slab_slots(max products, n) slots).  n_ctas large-column CTAs run at once: ws_bytes >=
+ *   n_ctas * 8 * slab slots.  Writes d_stats CHAOS / NNZ like pg_mcl_normalise.
+ * pg_mcl_compact: next CSC from the staging arrays: d_colptr_out = exclusive scan of d_kept (n + 1 entries),
+ *   rows / values copied; d_rows_out / d_vals_out hold d_stats[PG_MCL_STAT_NNZ] entries.
+ * pg_mcl_components: one root per column (the smallest index of its component) of the undirected graph with
+ *   an edge {i, j} per stored entry.
+ * d_stats: PG_MCL_STAT_WORDS int64, zeroed by the caller before pg_mcl_plan / pg_mcl_normalise.
+ * Scans use d_scan_ws of pg_mcl_scan_workspace_bytes(n) bytes.
+ */
+#define PG_MCL_PRUNE_THETA 1e-4f    /* theta: entries below it are pruned after expansion */
+#define PG_MCL_SELECT_S 1024        /* S: entries a column keeps at most                   */
+#define PG_MCL_CHAOS_TAU 1e-4f      /* tau: convergence when max chaos falls below it      */
+#define PG_MCL_MAX_ITER 100         /* T: iterations at most                               */
+#define PG_MCL_WARP_PRODUCTS 64     /* columns with at most this many products take the warp path */
+#define PG_MCL_SMEM_SLOTS 2048      /* accumulator slots a CTA keeps in shared memory      */
+#define PG_MCL_STAT_CHAOS 0
+#define PG_MCL_STAT_NNZ 1
+#define PG_MCL_STAT_PRODUCTS 2
+#define PG_MCL_STAT_MAXPROD 3
+#define PG_MCL_STAT_LARGE 4
+#define PG_MCL_STAT_WORDS 8
+int64_t pg_mcl_scan_workspace_bytes(int64_t n);
+int64_t pg_mcl_slab_slots(int64_t max_products, int64_t n);
+int pg_mcl_normalise(const int64_t *d_colptr, const int32_t *d_rows, float *d_vals, int64_t n, int64_t *d_stats,
+                     pg_stream_t stream);
+int pg_mcl_plan(const int64_t *d_colptr, const int32_t *d_rows, int64_t n, int64_t *d_prod, int64_t *d_stage_off,
+                int32_t *d_large, int64_t *d_stats, void *d_scan_ws, int64_t scan_ws_bytes, pg_stream_t stream);
+int pg_mcl_expand(const int64_t *d_colptr, const int32_t *d_rows, const float *d_vals, int64_t n, const int64_t *d_prod,
+                  const int64_t *d_stage_off, const int32_t *d_large, int64_t n_large, int64_t max_products, float inflation,
+                  int32_t *d_stage_rows, float *d_stage_vals, int64_t *d_kept, int64_t *d_stats, void *d_ws, int64_t ws_bytes,
+                  int n_ctas, pg_stream_t stream);
+int pg_mcl_compact(const int64_t *d_stage_off, const int32_t *d_stage_rows, const float *d_stage_vals, const int64_t *d_kept,
+                   int64_t n, int64_t *d_colptr_out, int32_t *d_rows_out, float *d_vals_out, void *d_scan_ws,
+                   int64_t scan_ws_bytes, pg_stream_t stream);
+int pg_mcl_components(const int64_t *d_colptr, const int32_t *d_rows, int64_t n, int32_t *d_root, pg_stream_t stream);
+
 /* ---- K8: per-record breakpoint labelling -------------------------------------------
  * Replaces seq2path_jit_ (:1523-1573): a hit matches when (code, v6) equals some
  * node's (code, v5) (Q7); matched hits are chained greedily ("starts[-1] < idx":

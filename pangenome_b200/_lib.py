@@ -8,6 +8,10 @@ LIB_PATH = os.path.join(HERE, "libpgdbg.so")
 
 PG_MODE_LITERAL, PG_MODE_LITERAL_RC, PG_MODE_CANONICAL = 0, 1, 2
 PG_STAT_OVERFLOW, PG_STAT_SHORT, PG_STAT_USED, PG_STAT_ENTRIES, PG_STAT_LOST, PG_STAT_WORDS = 0, 1, 2, 3, 4, 8
+# Markov clustering constants (include/pgdbg.h PG_MCL_*): theta, S, tau, T and the stats block layout
+PG_MCL_PRUNE_THETA, PG_MCL_SELECT_S, PG_MCL_CHAOS_TAU, PG_MCL_MAX_ITER = 1e-4, 1024, 1e-4, 100
+PG_MCL_WARP_PRODUCTS, PG_MCL_SMEM_SLOTS = 64, 2048
+PG_MCL_STAT_CHAOS, PG_MCL_STAT_NNZ, PG_MCL_STAT_PRODUCTS, PG_MCL_STAT_MAXPROD, PG_MCL_STAT_LARGE, PG_MCL_STAT_WORDS = 0, 1, 2, 3, 4, 8
 
 c_i64, c_int, c_vp = ctypes.c_int64, ctypes.c_int, ctypes.c_void_p
 
@@ -102,6 +106,14 @@ SIGNATURES = {
     "pg_graph_components": (c_int, [GT, ctypes.c_uint32, c_vp]),
     "pg_graph_export_edges": (c_int, [GT, PT, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp]),
     "pg_graph_export_nodes": (c_int, [GT, PT, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp]),
+    "pg_mcl_scan_workspace_bytes": (c_i64, [c_i64]),
+    "pg_mcl_slab_slots": (c_i64, [c_i64, c_i64]),
+    "pg_mcl_normalise": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp]),
+    "pg_mcl_plan": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "pg_mcl_expand": (c_int, [c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_i64, ctypes.c_float, c_vp, c_vp, c_vp, c_vp,
+                              c_vp, c_i64, c_int, c_vp]),
+    "pg_mcl_compact": (c_int, [c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "pg_mcl_components": (c_int, [c_vp, c_vp, c_i64, c_vp, c_vp]),
     "pg_label_workspace_bytes": (c_i64, [c_i64]),
     "pg_label_regions": (c_int, [GT, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp,
                                  c_i64, c_vp]),

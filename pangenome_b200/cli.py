@@ -7,7 +7,10 @@ flags such as ``-m`` are skipped exactly like upstream, F1), same ``# `` banner
 lines, same table rows, same side-file names.  ``-d`` / ``-D`` read tables in the
 reference's ``.npz`` layout; like upstream the dBG is saved to ``<input>_db.npz`` after stage 1
 (``--no-dump-db`` skips the file, the banners stay).  Extra long options (ignored by the reference's
-parser, so scripts stay portable): ``--min-edge-weight W``, ``--no-mcl-file``, ``--no-dump-db``.
+parser, so scripts stay portable): ``--min-edge-weight W``, ``--no-mcl-file``, ``--no-dump-db``, and
+``--cluster {components,mcl}`` with ``--inflation R``: the region labels come from the connected components of the
+edge list (the default) or from Markov clustering on the GPU with inflation R (default 1.5, what the reference passes
+to ``mcl -I``; R > 1) in place of the reference's external ``mcl`` run.  An existing ``<xyz>.mcl`` still wins.
 
 Multi-GPU: ``torchrun --nproc-per-node N kmer_b200.py -i input.fasta -k 27`` - every rank packs its
 record-aligned byte range of the one input file, the dBG is hash-partitioned across the GPUs
@@ -34,7 +37,7 @@ def manual_print(out=sys.stdout):
 
 def parse_args(argv):
     args = {'-i': '', '-k': '50', '-n': '2**63', '-r': '', '-d': '', '-R': '', '-D': '', '-c': '2'}
-    extra = {'--min-edge-weight': '1'}
+    extra = {'--min-edge-weight': '1', '--cluster': 'components', '--inflation': '1.5'}
     flags = set()
     N = len(argv)
     for i in range(1, N):
@@ -48,6 +51,20 @@ def parse_args(argv):
         elif k.startswith('--'):
             flags.add(k)
     return args, extra, flags
+
+
+def cluster_options(extra):
+    """(method, inflation) from ``--cluster`` / ``--inflation``; a bad value exits with a message."""
+    method = extra['--cluster']
+    if method not in ('components', 'mcl'):
+        raise SystemExit("pangenome_b200: --cluster must be 'components' or 'mcl', got %r" % method)
+    try:
+        r = float(extra['--inflation'])
+    except ValueError:
+        raise SystemExit("pangenome_b200: --inflation needs a number, got %r" % extra['--inflation'])
+    if not 1.0 < r < 64.0:
+        raise SystemExit("pangenome_b200: --inflation must be greater than 1 (and below 64), got %r" % extra['--inflation'])
+    return method, r
 
 
 def _eval_n(text):
@@ -91,6 +108,7 @@ def entry_point(argv, out=sys.stdout):
     if not qry:
         manual_print(out)
         raise SystemExit()
+    method, inflation = cluster_options(extra)
     if args['-R']:
         raise SystemExit("pangenome_b200: -R (resuming the edge-weight stage from a _rdb_brkpt.npz) is not supported by the "
                          "GPU path; -r (dBG checkpoint) is")
@@ -111,7 +129,8 @@ def entry_point(argv, out=sys.stdout):
         del kmer_dict
         p('# find fr')
         stages.seq2graph(qry, kmer=kmer, bits=5, Ns=Ns, rdbg_dict=rdbg_dict, rc=rc1, out=out,
-                         min_weight=int(extra['--min-edge-weight']), write_mcl='--no-mcl-file' not in flags)
+                         min_weight=int(extra['--min-edge-weight']), write_mcl='--no-mcl-file' not in flags,
+                         cluster_method=method, inflation=inflation)
         return 0
     p('# build the dBG')
     st = time()
@@ -137,7 +156,8 @@ def entry_point(argv, out=sys.stdout):
     st = time()
     rc1 = ((rc & 1) == 1)
     stages.seq2graph(qry, kmer=kmer, bits=5, Ns=Ns, rdbg_dict=rdbg_dict, rc=rc1, out=out,
-                     min_weight=int(extra['--min-edge-weight']), write_mcl='--no-mcl-file' not in flags)
+                     min_weight=int(extra['--min-edge-weight']), write_mcl='--no-mcl-file' not in flags,
+                     cluster_method=method, inflation=inflation)
     p('# finished in', time() - st, 'seconds')
     return 0
 

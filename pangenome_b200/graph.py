@@ -3,8 +3,9 @@
 Mirrors what the reference's ``seq2graph`` (kmer_numba.py:1853-1951) does after
 the rdBG exists, with the external ``mcl`` process replaced by an on-GPU
 union-find (connected components of the edge list, optionally restricted to
-edges of weight >= ``min_weight``).  The host only sizes buffers, orders the
-(small) component list and formats text.
+edges of weight >= ``min_weight``) or, opt-in, by Markov clustering on the GPU
+(``cluster="mcl"``, pangenome_b200/mcl.py).  The host only sizes buffers, orders
+the (small) cluster list and formats text.
 """
 import ctypes
 
@@ -46,6 +47,36 @@ def path_hits(packed, rd, n_rec, strand=0, cap=None):
         if n <= cap:
             return Hits(hg, hn, hr, hv, n, strand)
         cap = n + 1024
+
+
+def _no_nodes():
+    z = np.zeros(0, np.uint32)
+    return z, np.zeros(0, np.uint64), z, np.zeros(0, np.int64)
+
+
+def dense_order(code, v5):
+    """Node order ascending by (code, v5) (device sort): codes are < 5^27 < 2^63, so int64 order is the unsigned order."""
+    o1 = torch.argsort(v5, stable=True)
+    return o1[torch.argsort(code[o1], stable=True)]
+
+
+def rank_clusters(code, v5, root):
+    """(order, label per node in that order, cluster count): ``order`` = dense_order(code, v5); clusters are ranked
+    by (size descending, smallest (code, v5)).  Device sorts only."""
+    nn = int(code.numel())
+    dev = code.device
+    order = dense_order(code, v5)
+    if nn == 0:
+        return order, torch.zeros(0, dtype=torch.int64, device=dev), 0
+    roots_sorted = root[order]
+    uniq, inverse, counts = torch.unique(roots_sorted, return_inverse=True, return_counts=True)
+    rank = torch.arange(nn, device=dev)
+    first_idx = torch.full((uniq.numel(),), nn, dtype=torch.int64, device=dev).scatter_reduce_(0, inverse, rank, "amin")
+    c1 = torch.argsort(first_idx, stable=True)
+    comp_order = c1[torch.argsort(-counts[c1], stable=True)]          # (size desc, smallest node asc)
+    label_of_comp = torch.empty_like(comp_order)
+    label_of_comp[comp_order] = torch.arange(uniq.numel(), device=dev)
+    return order, label_of_comp[inverse], int(uniq.numel())          # labels per node, in (code, v5) order
 
 
 class RdbgGraph:
@@ -101,10 +132,42 @@ class RdbgGraph:
         return f(c0, np.uint64), f(v0, np.uint32), f(c1, np.uint64), f(v1, np.uint32), f(w, np.uint32)
 
     def components(self, rd, min_weight=1, to_host=True):
-        """K7 + component ordering.  Returns (nslot, code, v5, label) per graph node; label = rank
+        """K7 + cluster ordering.  Returns (nslot, code, v5, label) per graph node; label = rank
         of the node's component under (size descending, smallest (code, v5)).  The union-find is
         a kernel; the ordering uses device sorts; labels are written to the node table directly."""
         check(self.L.pg_graph_components(ctypes.byref(self.c), int(min_weight), _stream()), "pg_graph_components")
+        nodes = self._export_nodes(rd)
+        if nodes is None:
+            return _no_nodes()
+        nslot, code, v5, root = nodes
+        return self._label(nslot, code, v5, root, to_host)
+
+    def mcl(self, rd, min_weight=1, inflation=1.5, to_host=True):
+        """K7m: Markov clustering (pangenome_b200/mcl.py) of the live edges (node slot a, node slot b, weight), nodes
+        numbered densely in (code, v5) order.  Returns what components() returns; the run's per-iteration
+        statistics stay in ``self.mcl_result``."""
+        from . import mcl
+        nodes = self._export_nodes(rd)
+        if nodes is None:
+            return _no_nodes()
+        nslot, code, v5, _ = nodes
+        nn = int(nslot.numel())
+        order = dense_order(code, v5)
+        dense = torch.full((self.cap,), -1, dtype=torch.int64, device=nslot.device)
+        dense[nslot[order]] = torch.arange(nn, device=nslot.device)
+        ek = self.edge_keys
+        live = ek != -1                                                   # PG_EMPTY
+        ek = ek[live]
+        a, b = dense[(ek >> 32) & 0xFFFFFFFF], dense[ek & 0xFFFFFFFF]
+        w = self.edge_w[live].long()                                      # uint32 weights in an int32 tensor: < 2^31
+        self.mcl_result = mcl.markov_cluster(nn, a, b, w, inflation, min_weight)
+        root = torch.empty(nn, dtype=torch.int64, device=nslot.device)
+        root[order] = self.mcl_result.root.long()
+        return self._label(nslot, code, v5, root, to_host)
+
+    def _export_nodes(self, rd):
+        """(nslot, code, v5, union-find parent) of the nodes that appear in an edge, or None when there is none;
+        every node label is reset to -1."""
         nn, _ = self.counts()
         dev = self.stats.device
         nslot = torch.empty(max(nn, 1), dtype=torch.int32, device=dev)
@@ -117,23 +180,14 @@ class RdbgGraph:
         nn = int(d_n.item())          # nodes that appear in at least one edge (<= inserted node slots)
         self.node_label.fill_(-1)
         if nn == 0:
-            z = np.zeros(0, np.uint32)
-            return z, np.zeros(0, np.uint64), z, np.zeros(0, np.int64)
-        nslot, code, v5, root = nslot[:nn].long(), code[:nn], v5[:nn].long(), root[:nn].long()
-        # nodes ascending by (code, v5): codes are < 5^27 < 2^63, so int64 order is the unsigned order
-        o1 = torch.argsort(v5, stable=True)
-        order = o1[torch.argsort(code[o1], stable=True)]
-        roots_sorted = root[order]
-        uniq, inverse, counts = torch.unique(roots_sorted, return_inverse=True, return_counts=True)
-        rank = torch.arange(nn, device=dev)
-        first_idx = torch.full((uniq.numel(),), nn, dtype=torch.int64, device=dev).scatter_reduce_(0, inverse, rank, "amin")
-        c1 = torch.argsort(first_idx, stable=True)
-        comp_order = c1[torch.argsort(-counts[c1], stable=True)]          # (size desc, smallest node asc)
-        label_of_comp = torch.empty_like(comp_order)
-        label_of_comp[comp_order] = torch.arange(uniq.numel(), device=dev)
-        label_sorted = label_of_comp[inverse]                             # per node, in (code, v5) order
+            return None
+        return nslot[:nn].long(), code[:nn], v5[:nn].long(), root[:nn].long()
+
+    def _label(self, nslot, code, v5, root, to_host):
+        """Label every node with the rank of its cluster (``root`` = any id shared by exactly the nodes of one
+        cluster) and write the labels into the node table."""
+        order, label_sorted, self.n_components = rank_clusters(code, v5, root)
         self.node_label.index_put_((nslot[order],), label_sorted.to(torch.int32))
-        self.n_components = int(uniq.numel())
         if not to_host:
             return None
         # host copies, sorted by (label, code, v5) - the order the cluster file is written in
@@ -295,8 +349,19 @@ def labels_from_mcl(lines, xyz_edges):
     return lab
 
 
-def seq2graph_device(packed, rd, k, Ns=2 ** 63, rc=False, min_weight=1, mcl_lines=None):
-    """Stages 3-5 on the GPU.  ``rd`` = rdBG table from DbgTable.select_rdbg()."""
+def cluster_nodes(g, rd, min_weight=1, cluster="components", inflation=1.5):
+    """(nslot, code, v5, label) per graph node under the chosen clustering: "components" (K7, the default) or "mcl"
+    (K7m, Markov clustering with inflation ``inflation``)."""
+    if cluster == "components":
+        return g.components(rd, min_weight)
+    if cluster == "mcl":
+        return g.mcl(rd, min_weight, inflation)
+    raise ValueError("cluster must be 'components' or 'mcl', got %r" % (cluster,))
+
+
+def seq2graph_device(packed, rd, k, Ns=2 ** 63, rc=False, min_weight=1, mcl_lines=None, cluster="components", inflation=1.5):
+    """Stages 3-5 on the GPU.  ``rd`` = rdBG table from DbgTable.select_rdbg().  ``cluster``: "components" or "mcl"
+    (see cluster_nodes); an externally produced cluster file (``mcl_lines``) overrides either."""
     k = int(min(max(1, k), 27))
     n_rec = packed.record_prefix(Ns, 1)
     n_strands = 2 if rc else 1
@@ -307,7 +372,7 @@ def seq2graph_device(packed, rd, k, Ns=2 ** 63, rc=False, min_weight=1, mcl_line
         g.add_hits(h, n_strands)
     res = GraphResult()
     res.edges = g.edges(rd)
-    nslot, code, v5, label = g.components(rd, min_weight)
+    nslot, code, v5, label = cluster_nodes(g, rd, min_weight, cluster if mcl_lines is None else "components", inflation)
     if mcl_lines is not None:      # an externally produced cluster file wins (the "# the mcl has been ran" path)
         lab = labels_from_mcl(mcl_lines, res.edges)
         label = np.array([lab[(c, v)] for c, v in zip(code.tolist(), v5.tolist())], dtype=np.int64)

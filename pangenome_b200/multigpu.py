@@ -82,11 +82,13 @@ class _GlobalIndex:
         return np.diff(self.seq_off)
 
 
-def seq2graph_distributed(packed, table, k, world, rank, data, rc=False, min_weight=1, n_rec=None, mcl_lines=None):
+def seq2graph_distributed(packed, table, k, world, rank, data, rc=False, min_weight=1, n_rec=None, mcl_lines=None,
+                          cluster="components", inflation=1.5):
     """Stages 2-5 after a distributed dBG build (SURVEY 8e): every rank selects the rdBG members
     among ITS keys, the small rdBG tables are all-gathered into one full table per rank, each rank
     walks its own records (K5), the hits (a few % of the positions) are gathered in rank-independent
-    form (record, position, literal code, v5, v6) and rank 0 runs K6-K8 on them.
+    form (record, position, literal code, v5, v6) and rank 0 runs K6-K8 on them (with the clustering
+    ``cluster`` / ``inflation`` of graph.cluster_nodes).
     Returns (GraphResult, rows) on rank 0 and (None, None) elsewhere."""
     from . import engine, graph
     L = _lib.load()
@@ -160,7 +162,7 @@ def seq2graph_distributed(packed, table, k, world, rank, data, rc=False, min_wei
         g.add_hits(h, n_strands)
     res = graph.GraphResult()
     res.edges = g.edges(rd)
-    res.nodes = g.components(rd, min_weight)
+    res.nodes = graph.cluster_nodes(g, rd, min_weight, cluster if mcl_lines is None else "components", inflation)
     if mcl_lines is not None:      # an externally produced cluster file wins (the "# the mcl has been ran" path, :1908)
         nslot, code, v5, _ = res.nodes
         lab = graph.labels_from_mcl(mcl_lines, res.edges)

@@ -205,9 +205,11 @@ def dbg2rdbg(kmer_dict):
 
 
 def seq2graph(qry, kmer=13, bits=5, Ns=1e6, brkpt="./breakpoint_rdbg.npz", rdbg_dict=None, saved=None, hashfunc=None,
-              jit=True, chunk=2 ** 33, rc=False, cluster=True, min_weight=1, out=None, write_mcl=True):
-    """Stages 3-5: edge weights -> ``<qry>_rdbg_weight.xyz``; components (or an existing
-    ``.xyz.mcl`` cluster file) -> labels; region table on ``out`` (stdout)."""
+              jit=True, chunk=2 ** 33, rc=False, cluster=True, min_weight=1, out=None, write_mcl=True,
+              cluster_method="components", inflation=1.5):
+    """Stages 3-5: edge weights -> ``<qry>_rdbg_weight.xyz``; clusters (connected components, or Markov clustering
+    with ``cluster_method="mcl"`` and ``inflation``; an existing ``.xyz.mcl`` cluster file wins) -> labels; region
+    table on ``out`` (stdout)."""
     out = out or sys.stdout
     kmer = min(max(1, int(kmer)), 27)
     packed, data = rdbg_dict.packed, rdbg_dict.data
@@ -226,7 +228,7 @@ def seq2graph(qry, kmer=13, bits=5, Ns=1e6, brkpt="./breakpoint_rdbg.npz", rdbg_
         import torch.distributed as dist
         n_rec = builder.global_record_prefix(packed, Ns, 1, world)
         res, rows = multigpu.seq2graph_distributed(packed, rdbg_dict.table, kmer, world, rank, data, rc=bool(rc), min_weight=min_weight,
-                                                   n_rec=n_rec, mcl_lines=mcl_lines)
+                                                   n_rec=n_rec, mcl_lines=mcl_lines, cluster=cluster_method, inflation=inflation)
         if rank == 0:
             res.write_xyz(oname)
             if mcl_lines is None and write_mcl:
@@ -234,7 +236,8 @@ def seq2graph(qry, kmer=13, bits=5, Ns=1e6, brkpt="./breakpoint_rdbg.npz", rdbg_
             out.write("".join("%s\t%d\t%d\t%s\t%d\n" % r for r in rows))
         dist.barrier()
         return LabelDict(res.nodes[1], res.nodes[2], res.nodes[3]) if rank == 0 else None
-    res = graph.seq2graph_device(packed, rdbg_dict.table, kmer, Ns=Ns, rc=bool(rc), min_weight=min_weight, mcl_lines=mcl_lines)
+    res = graph.seq2graph_device(packed, rdbg_dict.table, kmer, Ns=Ns, rc=bool(rc), min_weight=min_weight, mcl_lines=mcl_lines,
+                                 cluster=cluster_method, inflation=inflation)
     res.write_xyz(oname)
     if mcl_lines is None and write_mcl:
         res.write_mcl(oname + ".mcl")
