@@ -14,6 +14,8 @@ constexpr uint32_t PG_MAX_PROBE = 1u << 16;
 // whole table when 0), so a region of a table built in shared memory (region_build.cu) holds ALL the keys that hash into it.
 // hmask: region tables round the home slot down to a group of PG_REGION_GROUP slots (K3s reads a whole group per probe
 // step), so the linear-probing invariant "no free slot between home and the key" is stated from the group's first slot.
+// Region semantics hold whenever 0 < region_bits <= log2(capacity): a table of exactly ONE region is built by K3s / K3s-c
+// like any other, so every later upsert must start from the same group-aligned home (tests/test_table_geometry.py).
 #define PG_REGION_GROUP 4
 // hkind: which code the placement hash is taken of (pg_table.hash_kind): 0 = the base-5 key itself, 1 = its 2-bit form
 // (tables built from compact records, compact_build.cu; generic upserts and look-ups then pay a base-5 -> 2-bit conversion)
@@ -27,8 +29,9 @@ __host__ __device__ __forceinline__ uint64_t tv_home(const TableView &t, uint64_
 inline TableView make_view(const pg_table *t) {
     int bits = 0; while ((1ll << bits) < t->capacity) bits++;
     const uint64_t capmask = (uint64_t)t->capacity - 1;
-    const uint64_t rmask = (t->region_bits > 0 && t->region_bits < bits) ? ((1ull << t->region_bits) - 1ull) : capmask;
-    const uint64_t hmask = rmask != capmask ? ~(uint64_t)(PG_REGION_GROUP - 1) : ~0ull;
+    const bool region = t->region_bits > 0 && t->region_bits <= bits;
+    const uint64_t rmask = region ? ((1ull << t->region_bits) - 1ull) : capmask;
+    const uint64_t hmask = region ? ~(uint64_t)(PG_REGION_GROUP - 1) : ~0ull;
     return TableView{t->d_slots, capmask, t->d_stats, 64 - bits, pg_tag(t), rmask, hmask, t->hash_kind ? 1 : 0, t->k};
 }
 
