@@ -281,7 +281,8 @@ typedef struct pg_cbuckets {
      * mix64(2-bit code), bits = log2(ranks); bucket o is stored straight into rank o's receive buffers over NVLink at the
      * slice of source rank my_rank - compact records at d_peer_bases[o] + my_rank * part_cap, wide ones at
      * d_wide_peer_bases[o] + my_rank * wide_cap (records).  d_records / d_wide stay NULL.  What arrived is split into
-     * hash-prefix buckets by pg_records_split_c and the wide segments are upserted by pg_wide_insert. */
+     * hash-prefix buckets by pg_records_split_c (out->bits 0..10; 0 = one bucket, for a table of one region per rank)
+     * and the wide segments are upserted by pg_wide_insert. */
     uint64_t *const *d_peer_bases;
     uint64_t *const *d_wide_peer_bases;
     int32_t my_rank, reserved2;

@@ -255,6 +255,8 @@ class RoundBuilder:
                                                   self.owner_bits, 0, rank, 0))
             self.wire_seg_off = torch.arange(W, dtype=torch.int64, device=dev) * cw
             self.sent_total = torch.zeros(W, dtype=torch.int64, device=dev)
+            # per source: the most records one round of this build sent to this rank, surplus over cap_wire included
+            self.wire_peak = torch.zeros(W, dtype=torch.int64, device=dev)
             self._arriving = W * cw
             # the same receive buffers under compact records: W segments of cw 8-byte records, then W segments of cw / 2
             # wide (16-byte) records; counters [W compact | W wide]
@@ -377,6 +379,8 @@ class RoundBuilder:
             self._configure(self._next_capacity or self.table.capacity)
         self._next_capacity, self._reconfigure = None, False
         self.table.clear()
+        if self.world > 1:
+            self.wire_peak.zero_()
         self._begun = True
 
     def build_async(self, packed, n_rec=None, ev=None):
@@ -458,6 +462,7 @@ class RoundBuilder:
                     x0 = stamp(B)
                     # one all-to-all for both counters: [owner][compact, wide] -> [source][compact, wide]
                     recv_c, recv_w = exchange_record_counts(self.csend_counts[i], self.crecv[i], W)
+                    torch.maximum(self.wire_peak, recv_c, out=self.wire_peak)
                     self._ev_a2a = torch.cuda.Event()
                     self._ev_a2a.record(B)
                     x1 = stamp(B)
@@ -472,6 +477,7 @@ class RoundBuilder:
                     bs = self.sets[0]
                     x0 = stamp(B)
                     dist.all_to_all_single(self.recv_counts[i], self.send_counts[i][:W])
+                    torch.maximum(self.wire_peak, self.recv_counts[i], out=self.wire_peak)
                     self._ev_a2a = torch.cuda.Event()
                     self._ev_a2a.record(B)
                     x1 = stamp(B)
@@ -574,6 +580,14 @@ class RoundBuilder:
         if self.adaptive:
             self.retune()
 
+    def wire_records_peak(self):
+        """The most records one source sent to one owner in one round of the last build, over all ranks (a collective).
+        Above cap_wire, the records past the owner's receive segment were lost on the wire (or, on compact records,
+        went to its wide segment)."""
+        p = self.wire_peak.max().reshape(1)
+        dist.all_reduce(p, op=dist.ReduceOp.MAX)
+        return int(p.item())
+
     def retune(self, load=0.5):
         """Shared-memory region build: size the table for the NEXT build of this builder from the distinct keys the last one
         found (load <= ``load``; a serving loop sees inputs of one kind).  A K3s launch writes every slot of the table it
@@ -634,11 +648,11 @@ def build_table(packed, k, rc=True, Ns=2 ** 63, mode=None, world=1, rank=0, capa
     strands = 1 if mode == _lib.PG_MODE_LITERAL else 2
     n_rec = global_record_prefix(packed, Ns, strands, world)
     n_bases = int(packed.seq_off[n_rec] - packed.seq_off[0]) if n_rec > 0 else 0
-    spill_frac = 1.0 / 16
+    spill_frac, slack = 1.0 / 16, 1.25
     err = None
     for _ in range(max_attempts + 1):
         b = RoundBuilder(k, mode, max(n_bases, 1), world=world, rank=rank, device=packed.pk2.device, capacity=capacity, rounds=rounds,
-                         spill_frac=spill_frac, region_bits=region_bits, sample=sample, compact=compact)
+                         slack=slack, spill_frac=spill_frac, region_bits=region_bits, sample=sample, compact=compact)
         b.adaptive = False              # one build: nothing to retune for
         b.begin()
         b.build_async(packed, n_rec)
@@ -650,6 +664,16 @@ def build_table(packed, k, rc=True, Ns=2 ** 63, mode=None, world=1, rank=0, capa
             err = e
             if b.compact:           # positions the compact records cannot hold overflowed the wide spill: 16-byte records
                 compact = False
+            elif world > 1:
+                # across GPUs: a wire bucket (R / W * slack + 8192 records per source and owner) overflows when one owner
+                # takes more than its share of a round - a hot key such as a long poly-A - and a local bucket when one
+                # hash prefix does.  Either share stays the same however the stream is cut into rounds, so more rounds do
+                # not help; a wider wire bucket (at slack W it holds a whole round) or a larger local spill does
+                peak = b.wire_records_peak()
+                if peak > b.cap_wire and slack < world:
+                    slack = min(float(world), max(2 * slack, 1.05 * (peak - 8192) * world / b.round_len))
+                else:
+                    spill_frac = min(1.0, spill_frac * 4)
             else:
                 rounds, spill_frac = 4 * b.n_rounds, min(1.0, spill_frac * 4)
         except TableFull as e:

@@ -341,7 +341,10 @@ k2c_multisplit_c(CSplitArgs a) {
     }
     __syncthreads();
     const uint32_t n_tiles = s_tile0[n_seg];
-    const int shift = 64 - (SLICED ? a.in.bits : 0) - a.bits;
+    // K2b-c into one bucket (a one-region table per rank: a.bits == 0) would shift by 64, which is undefined; the fan
+    // mask of 0 sends every record to bucket 0 whatever the shift, so it is clamped to 63
+    const int shift_ = 64 - (SLICED ? a.in.bits : 0) - a.bits;
+    const int shift = shift_ < 64 ? shift_ : 63;
 
     int seg = 0;
     for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -749,8 +752,8 @@ extern "C" int pg_records_split_c(const pg_cbuckets *in, const pg_cbuckets *out,
     CSplitArgs a;
     int rc = make_cbuckets(in, "pg_records_split_c", a.in); if (rc) return rc;
     rc = make_cbuckets(out, "pg_records_split_c", a.out); if (rc) return rc;
-    if (a.in.peers || a.out.peers || in->bits > 6 || out->bits < 1 || out->bits > 10 || k < 1 || k > 27 || in->d_records == out->d_records)
-        return pg_fail(PG_ERR_INVALID, "pg_records_split_c: bad geometry (local sets, <= 64 segments, 2..1024 buckets, distinct buffers)");
+    if (a.in.peers || a.out.peers || in->bits > 6 || out->bits < 0 || out->bits > 10 || k < 1 || k > 27 || in->d_records == out->d_records)
+        return pg_fail(PG_ERR_INVALID, "pg_records_split_c: bad geometry (local sets, <= 64 segments, 1..1024 buckets, distinct buffers)");
     cudaStream_t st = (cudaStream_t)stream_;
     PG_CUDA(cudaMemsetAsync(out->d_counts, 0, (size_t)(1ll << out->bits) * 8, st));
     a.bits = out->bits; a.k = k; a.stats = d_table_stats; a.sliced = 0;

@@ -3,6 +3,12 @@ record-aligned byte range (pangenome_b200/shard.py) - equals the oracle on the w
 checksum, rdBG key set, .xyz lines in file order, region rows; then the same through the drop-in CLI.
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29533 tests/mg_check.py
+
+With --one-device every rank runs on cuda:0 and the ranks talk over gloo (NCCL refuses two ranks on one device).  The
+builder cannot tell: the peer stores go through CUDA IPC between processes of one device, and a gloo collective on CUDA
+tensors reads its input after the current stream's work and returns only when every rank's input has arrived, so the
+count exchange still orders the peer stores.  This mode also runs the CLI with --cluster mcl against a one-GPU run.
+tests/test_gpu_multi_one_device.py starts it without torchrun, with the process group already set up.
 """
 import io
 import os
@@ -29,11 +35,20 @@ def files(world):
     yield "plant-like 8 x 300 kb", synth.plant_like(n_genomes=8, length=300_000, n_chrom=5, n_families=50), 27
 
 
-def main():
-    rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
-    torch.cuda.set_device(local)
-    dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    from pangenome_b200 import _lib, builder, cli, engine, measure, multigpu, shard
+def main(argv=None):
+    argv = sys.argv[1:] if argv is None else argv
+    one_device = "--one-device" in argv
+    rank, world = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"])
+    if one_device:
+        os.environ["LOCAL_RANK"] = "0"              # the CLI selects its device from LOCAL_RANK
+        torch.cuda.set_device(0)
+        if not dist.is_initialized():
+            dist.init_process_group("gloo")
+    else:
+        local = int(os.environ["LOCAL_RANK"])
+        torch.cuda.set_device(local)
+        dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    from pangenome_b200 import _lib, builder, cli, engine, graph, measure, multigpu, shard
     import oracle
     for name, data, k in files(world):
         cuts = shard.cut_points(data, world)
@@ -93,6 +108,23 @@ def main():
             z = np.load(path + "_db.npz")
             assert int(z["parameters"][2]) == ref["dbg"][0].size, "CLI _db.npz entry count differs"
             print("mg_check ok: CLI %s under torchrun: %d rows, %d edges" % (name, len(got), len(full["xyz"])), flush=True)
+        if one_device:
+            # --cluster mcl: K7m runs on rank 0 over the gathered edges; cluster file and rows equal a one-GPU run
+            mpath = os.path.join(tmp[0], "mcl.fa")
+            if rank == 0:
+                with open(mpath, "wb") as f:
+                    f.write(data)
+            dist.barrier()
+            out = io.StringIO()
+            cli.entry_point(["prog", "-i", mpath, "-k", str(k), "--cluster", "mcl", "--no-dump-db"], out=out)
+            if rank == 0:
+                whole = engine.PackedSeqs(engine.to_device_bytes(data))
+                t1, _ = engine.build_dbg(whole, k)
+                one = graph.seq2graph_device(whole, t1.select_rdbg(), k, cluster="mcl")
+                got = [l for l in out.getvalue().splitlines() if l and not l.startswith("#")]
+                assert got == ["%s\t%d\t%d\t%s\t%d" % r for r in one.rows(whole, data)], "CLI --cluster mcl rows differ"
+                assert open(mpath + "_rdbg_weight.xyz.mcl").read().split("\n")[:-1] == one.mcl_lines(), "CLI .mcl differs"
+                print("mg_check ok: CLI --cluster mcl %s: %d rows, %d clusters" % (name, len(got), len(one.mcl_lines())), flush=True)
         dist.barrier()
     dist.barrier()
     dist.destroy_process_group()
