@@ -40,6 +40,8 @@ extern "C" {
 #define PG_ERR_CUDA (-2)       /* a CUDA runtime call failed */
 #define PG_ERR_WORKSPACE (-3)  /* workspace too small */
 #define PG_ERR_CAPACITY (-4)   /* an output buffer / table is too small */
+#define PG_ERR_NOT_BGZF (-5)   /* pg_host_bgzf_index: the file does not start with a BGZF member */
+#define PG_ERR_INFLATE (-6)    /* pg_bgzf_inflate: a member failed to decode (see its d_status) */
 
 #define PG_MODE_LITERAL 0      /* one strand, literal keys            (-c 0 / -c 1)       */
 #define PG_MODE_LITERAL_RC 1   /* both strands, two literal inserts per position (-c 2/3) */
@@ -113,6 +115,42 @@ int pg_fasta_scan_pack(const uint8_t *d_fasta, int64_t nbytes,
                        uint32_t *d_pk2, uint32_t *d_amb, int64_t cap_bases,
                        int64_t *d_hdr_off, int64_t *d_seq_off, int64_t cap_records,
                        int64_t *d_counts, void *d_ws, int64_t ws_bytes, pg_stream_t stream);
+
+/* ---- BGZF input: gzip members of at most 64 KiB, each a self-contained raw-DEFLATE stream -------
+ * (the `bgzip` / `samtools faidx` format: gzip header with FLG = FEXTRA and a "BC" extra subfield of
+ * SLEN 2 holding BSIZE = member size - 1; CRC-32 and ISIZE trailer).  A concatenation of BGZF files is
+ * BGZF too (its empty EOF marker members then appear mid-file).
+ * pg_host_bgzf_index (HOST pointers): walks the member headers of the file image gz[nbytes];
+ *   member_off[i] = byte offset of member i in the file, out_off[i] = offset of its output in the
+ *   inflated stream (exclusive scan of ISIZE); both need cap + 1 entries, entry n_members holds the
+ *   file size / the inflated size.  counts[0] = n_members (may exceed cap: then only the first cap
+ *   entries were written - grow and call again), counts[1] = inflated size.  Returns PG_ERR_NOT_BGZF
+ *   when the first member is not BGZF (plain text, a `gzip` file, an empty file), PG_ERR_INVALID when
+ *   a later member is not BGZF, is truncated, or claims more than 65536 output bytes.
+ * pg_bgzf_inflate: inflates members [0, n_members) of d_gz[gz_bytes] into d_out[out_bytes] in ONE
+ *   launch, member i from d_gz[d_member_off[i], d_member_off[i + 1]) into
+ *   d_out[d_out_off[i], d_out_off[i + 1]) (device arrays of n_members + 1 entries: the index above,
+ *   or any contiguous slice of it rebased to its first entry).  Every member is checked: header,
+ *   Huffman codes, back-reference distances, output length = ISIZE = its window, CRC-32.  A bad
+ *   member never makes the kernel read or write outside its own input and output ranges.
+ *   d_status (device, 2 int64, overwritten): [0] = members that failed, [1] = (first failed member
+ *   << 8) | its PG_INF_ERR_* kind, INT64_MAX when none failed.  Returns without synchronising: the
+ *   caller reads d_status before it uses d_out.
+ */
+#define PG_INF_ERR_HEADER 1     /* not a BGZF member header, or its window does not fit */
+#define PG_INF_ERR_TRUNCATED 2  /* the compressed data ends inside a block */
+#define PG_INF_ERR_BLOCK 3      /* block type 3 */
+#define PG_INF_ERR_STORED 4     /* stored block: LEN and NLEN disagree */
+#define PG_INF_ERR_CODE 5       /* bad code lengths: over-subscribed or incomplete code, bad repeat, too many symbols */
+#define PG_INF_ERR_SYMBOL 6     /* a bit pattern no code word matches, or literal/length 286-287, distance 30-31 */
+#define PG_INF_ERR_DISTANCE 7   /* a back-reference before the start of the member's output */
+#define PG_INF_ERR_OVERFLOW 8   /* more output than ISIZE */
+#define PG_INF_ERR_LENGTH 9     /* less output than ISIZE, ISIZE != window, or bytes left after the final block */
+#define PG_INF_ERR_CRC 10       /* CRC-32 of the output differs from the trailer's */
+int pg_host_bgzf_index(const uint8_t *gz, int64_t nbytes, int64_t *member_off, int64_t *out_off, int64_t cap,
+                       int64_t *counts);
+int pg_bgzf_inflate(const uint8_t *d_gz, int64_t gz_bytes, const int64_t *d_member_off, const int64_t *d_out_off,
+                    int64_t n_members, uint8_t *d_out, int64_t out_bytes, int64_t *d_status, pg_stream_t stream);
 
 /* ---- K2+K3: k-mer extraction fused with table insertion ---------------------
  * pg_table_clear  : all slots empty (for every epoch), stats zero: 16 B/slot of HBM writes

@@ -10,6 +10,11 @@ PG_MODE_LITERAL, PG_MODE_LITERAL_RC, PG_MODE_CANONICAL = 0, 1, 2
 PG_STAT_OVERFLOW, PG_STAT_SHORT, PG_STAT_USED, PG_STAT_ENTRIES, PG_STAT_LOST, PG_STAT_WORDS = 0, 1, 2, 3, 4, 8
 # Markov clustering constants (include/pgdbg.h PG_MCL_*): theta, S, tau, T and the stats block layout
 PG_MCL_PRUNE_THETA, PG_MCL_SELECT_S, PG_MCL_CHAOS_TAU, PG_MCL_MAX_ITER = 1e-4, 1024, 1e-4, 100
+# BGZF input (include/pgdbg.h): "not BGZF" return code and the member error kinds d_status reports
+PG_ERR_NOT_BGZF = -5
+PG_INF_ERRORS = {1: "bad header", 2: "truncated deflate data", 3: "invalid block type", 4: "stored block length check",
+                 5: "invalid code lengths", 6: "invalid code", 7: "distance too far back", 8: "more output than ISIZE",
+                 9: "length mismatch", 10: "CRC-32 mismatch"}
 PG_MCL_WARP_PRODUCTS, PG_MCL_SMEM_SLOTS = 64, 2048
 PG_MCL_STAT_CHAOS, PG_MCL_STAT_NNZ, PG_MCL_STAT_PRODUCTS, PG_MCL_STAT_MAXPROD, PG_MCL_STAT_LARGE, PG_MCL_STAT_WORDS = 0, 1, 2, 3, 4, 8
 
@@ -96,6 +101,8 @@ SIGNATURES = {
     "pg_hits_rekey": (c_int, [PT, c_vp, c_vp, c_i64, c_vp, c_vp]),
     "pg_host_write_xyz": (c_int, [ctypes.c_char_p, c_vp, c_vp, c_vp, c_vp, c_vp, c_i64]),
     "pg_host_write_mcl": (c_int, [ctypes.c_char_p, c_vp, c_vp, c_vp, c_i64]),
+    "pg_host_bgzf_index": (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_vp]),
+    "pg_bgzf_inflate": (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp]),
     "pg_host_oakht_capacity": (c_i64, [c_i64]),
     "pg_host_build_oakht": (c_int, [c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "pg_path_workspace_bytes": (c_i64, [c_i64]),

@@ -12,6 +12,10 @@ parser, so scripts stay portable): ``--min-edge-weight W``, ``--no-mcl-file``, `
 edge list (the default) or from Markov clustering on the GPU with inflation R (default 1.5, what the reference passes
 to ``mcl -I``; R > 1) in place of the reference's external ``mcl`` run.  An existing ``<xyz>.mcl`` still wins.
 
+Input: plain FASTA, or FASTA compressed by ``bgzip`` (BGZF: its members are inflated on the GPU) or by ``gzip``
+(inflated on the host).  Side files keep the name given with ``-i`` (``input.fa.gz_rdbg_weight.xyz``, ``input.fa.gz_db.npz``);
+``-r`` checkpoint offsets are positions in the decompressed stream.
+
 Multi-GPU: ``torchrun --nproc-per-node N kmer_b200.py -i input.fasta -k 27`` - every rank packs its
 record-aligned byte range of the one input file, the dBG is hash-partitioned across the GPUs
 (pangenome_b200/builder.py), rank 0 prints the table and writes the side files.

@@ -41,9 +41,51 @@ def cut_points(buf, world):
     return cuts
 
 
-def read_rank_range(path, world, rank):
-    """(bytes of this rank's record-aligned range, (begin, end), file size).  Only the rank's own pages are read
-    (plus the few a cut search touches)."""
+def member_rank_range(out_off, world, rank, inflate):
+    """The cut rule above applied to the INFLATED stream of a file of independently compressed members (BGZF), reading
+    only the members around this rank's range.  ``out_off``: the n + 1 offsets of the members' output in the inflated
+    stream (exclusive scan of their sizes); ``inflate(i0, i1)``: the inflated bytes of members [i0, i1).  The search
+    starts at the member holding byte nominal_r - 1 and extends in doubling batches of members until the cut after
+    nominal_{r+1} is found or the file ends.  Returns what read_rank_range returns, with the inflated size for the
+    file size."""
+    import bisect
+    n, size = len(out_off) - 1, int(out_off[-1])
+    if size == 0:
+        return b"", (0, 0), 0
+    lo, hi = rank * size // world, (rank + 1) * size // world
+    first = bisect.bisect_right(out_off, max(lo - 1, 0)) - 1         # the member holding that byte (empty ones skipped)
+    base, end, batch = int(out_off[first]), first, 1
+    buf = bytearray()
+
+    def grow():
+        nonlocal end, batch
+        nxt = min(n, end + batch)
+        buf.extend(inflate(end, nxt))
+        end, batch = nxt, 2 * batch
+
+    def cut(nominal):
+        if nominal <= 0:
+            return 0
+        if nominal >= size:
+            return size
+        pos = nominal - 1 - base
+        while True:
+            j = buf.find(b"\n>", pos)
+            if j >= 0:
+                return base + j + 1
+            if end == n:
+                return size
+            pos = max(pos, len(buf) - 1)
+            grow()
+
+    a, b = cut(lo), cut(hi)
+    while base + len(buf) < b:         # the last rank's range runs to the end of the file
+        grow()
+    return bytes(buf[a - base:b - base]), (a, b), size
+
+
+def plain_rank_range(path, world, rank):
+    """read_rank_range of an uncompressed file: only the rank's own pages are read (plus the few a cut search touches)."""
     size = os.path.getsize(path)
     if size == 0:
         return b"", (0, 0), 0
@@ -56,3 +98,10 @@ def read_rank_range(path, world, rank):
         finally:
             mm.close()
     return data, (a, b), size
+
+
+def read_rank_range(path, world, rank):
+    """(bytes of this rank's record-aligned range of the decompressed input, (begin, end), decompressed size).  The
+    input may be plain FASTA or gzip / BGZF compressed (pangenome_b200/seqfile.py)."""
+    from . import seqfile
+    return seqfile.read_rank_range(path, world, rank)

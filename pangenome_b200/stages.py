@@ -22,11 +22,10 @@ class DbgHandle:
 
 
 def _read(qry):
-    """The whole file as a read-only uint8 view of its page-cache pages (np.memmap: nothing is copied on the host; the
-    H2D copy streams straight out of the mapping)."""
-    if os.path.getsize(qry) == 0:
-        return np.zeros(0, dtype=np.uint8)
-    return np.memmap(qry, dtype=np.uint8, mode="r")
+    """(host bytes, device bytes) of the whole input, decompressed when it is gzip / BGZF (seqfile.load).  Plain FASTA
+    stays a read-only np.memmap on the host: nothing is copied there, the H2D copy streams straight out of the mapping."""
+    from . import seqfile
+    return seqfile.load(qry)
 
 
 def _dist_env():
@@ -41,9 +40,10 @@ def _dist_env():
 
 
 def seq_chk(qry):
-    """kmer_numba.py:873-886: peek 40 bytes, '>' anywhere at a line start -> fasta."""
-    with open(qry, "rb") as f:
-        s = f.read(40)
+    """kmer_numba.py:873-886: peek 40 bytes, '>' anywhere at a line start -> fasta.  The bytes are those of the
+    decompressed stream when the file is gzip / BGZF compressed."""
+    from . import seqfile
+    s = seqfile.head(qry, 40)
     if s[:1] == b">" or b"\n>" in s:
         return "fasta"
     if s[:1] == b"@" or b"\n@" in s:
@@ -63,6 +63,7 @@ def seq2rdbg(qry, kmer=13, bits=5, Ns=1e6, chunk=2 ** 32, brkpt="./breakpoint", 
         raise ValueError("only the reference's base-5 code (bits=5) is supported")
     kmer = min(max(1, int(kmer)), 27)
     world, rank = _dist_env()
+    d_bytes = None
     if data is None:
         if seq_chk(qry) != "fasta":
             raise SystemExit("pangenome_b200: %s is not FASTA (the reference's fastq branch is broken upstream)" % qry)
@@ -71,8 +72,8 @@ def seq2rdbg(qry, kmer=13, bits=5, Ns=1e6, chunk=2 ** 32, brkpt="./breakpoint", 
             data, _, _ = shard.read_rank_range(qry, world, rank)
             data = np.frombuffer(data, dtype=np.uint8)
         else:
-            data = _read(qry)
-    packed = engine.PackedSeqs(engine.to_device_bytes(data))
+            data, d_bytes = _read(qry)
+    packed = engine.PackedSeqs(d_bytes if d_bytes is not None else engine.to_device_bytes(data))
     strands = 2 if rc else 1
     resume = bool(brkpt) and os.path.isfile(brkpt)
     from . import builder
@@ -189,8 +190,8 @@ def load_dbg(qry, fn, kmer):
     """``-d`` / ``-D``: a table saved by the reference (or by ``dump``) + the packed input."""
     from . import npz
     kmer = min(max(1, int(kmer)), 27)
-    data = _read(qry)
-    packed = engine.PackedSeqs(engine.to_device_bytes(data))
+    data, d_bytes = _read(qry)
+    packed = engine.PackedSeqs(d_bytes)
     table = npz.load(fn, kmer, device=packed.pk2.device)
     return DbgHandle(table, packed, data, packed.n_rec)
 

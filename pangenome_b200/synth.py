@@ -4,6 +4,9 @@
 All sets: uppercase ACGT only, ``>g{g} synthetic`` headers, 80-column LF lines,
 trailing newline.
 """
+import struct
+import zlib
+
 import numpy as np
 
 _ACGT = np.frombuffer(b"ACGT", dtype=np.uint8)
@@ -139,3 +142,33 @@ def n_kmer_insertions(seq_lengths, k, rc=True):
     """The metric's unit (BASELINE.md section 3): 2 * sum max(n - k + 1, 1)."""
     tot = sum(max(int(n) - k + 1, 1) for n in seq_lengths)
     return tot * (2 if rc else 1)
+
+
+# the empty member every BGZF file ends with (SAM/BAM specification 4.1.2)
+BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
+
+
+def bgzf_member(chunk, level=6, strategy=zlib.Z_DEFAULT_STRATEGY):
+    """One BGZF member (gzip header with the BC extra subfield, raw DEFLATE, CRC-32, ISIZE) holding ``chunk``."""
+    c = zlib.compressobj(level, zlib.DEFLATED, -15, 8, strategy)
+    d = c.compress(chunk) + c.flush()
+    bsize = 12 + 6 + len(d) + 8
+    if bsize > 65536:
+        raise ValueError("a BGZF member holds at most 65536 bytes: %d input bytes compressed to a %d-byte member" % (len(chunk), bsize))
+    return (b"\x1f\x8b\x08\x04\x00\x00\x00\x00\x00\xff\x06\x00BC\x02\x00" + struct.pack("<H", bsize - 1) + d
+            + struct.pack("<II", zlib.crc32(chunk), len(chunk)))
+
+
+def bgzf_bytes(data, block=65280, level=6, strategy=zlib.Z_DEFAULT_STRATEGY):
+    """``data`` as a BGZF file (what ``bgzip`` writes): members of ``block`` input bytes, then the 28-byte EOF member.
+    Large inputs are compressed by a thread pool (zlib releases the GIL)."""
+    data = bytes(data)
+    chunks = [data[i:i + block] for i in range(0, len(data), block)]
+    if len(chunks) > 64:
+        import os
+        from concurrent.futures import ThreadPoolExecutor
+        with ThreadPoolExecutor(min(32, os.cpu_count() or 1)) as ex:
+            members = list(ex.map(lambda c: bgzf_member(c, level, strategy), chunks))
+    else:
+        members = [bgzf_member(c, level, strategy) for c in chunks]
+    return b"".join(members) + BGZF_EOF
