@@ -116,6 +116,28 @@ int pg_fasta_scan_pack(const uint8_t *d_fasta, int64_t nbytes,
                        int64_t *d_hdr_off, int64_t *d_seq_off, int64_t cap_records,
                        int64_t *d_counts, void *d_ws, int64_t ws_bytes, pg_stream_t stream);
 
+/* ---- FASTQ pack: pg_fasta_scan_pack's outputs from a FASTQ file -----------------------------------
+ * A FASTQ record is exactly four lines: header ('@'), sequence, separator ('+'), quality (as long as the
+ * sequence line; never read otherwise).  The file F is packed as the FASTA file fasta(F) - each record's
+ * header line with '>' for '@', then its sequence line - would be by pg_fasta_scan_pack: same d_pk2 / d_amb,
+ * d_seq_off, d_counts[0..1]; d_hdr_off[r] = offset of record r's '@' line in F; d_counts[2] = '\n' count of F.
+ * Every byte of a sequence line but its '\n' is a base ('\r' too, Q9).  Lines of '\n' alone may follow the
+ * last record.  cap_records as for pg_fasta_scan_pack: d_counts[0] > cap_records means the index did not
+ * fit (grow and call again; d_status is then not set).  The workspace size depends on cap_records.
+ * d_status (2 int64, device): {-1, 0} for a valid file; otherwise {byte offset of the first malformed
+ * record's header line, PG_FQ_BAD_*} and d_counts[0] = d_counts[1] = 0, so nothing is built from it.
+ * The input is untrusted: any bytes give a status, never an out-of-bounds access.
+ */
+#define PG_FQ_BAD_HEADER 1         /* the header line does not start with '@' */
+#define PG_FQ_BAD_SEPARATOR 2      /* the separator line does not start with '+' */
+#define PG_FQ_BAD_QUALITY_LENGTH 3 /* quality and sequence lines differ in length */
+#define PG_FQ_TRUNCATED 4          /* the last record has fewer than four lines (e.g. wrapped FASTQ) */
+int64_t pg_fastq_workspace_bytes(int64_t nbytes, int64_t cap_records);
+int pg_fastq_scan_pack(const uint8_t *d_fastq, int64_t nbytes,
+                       uint32_t *d_pk2, uint32_t *d_amb, int64_t cap_bases,
+                       int64_t *d_hdr_off, int64_t *d_seq_off, int64_t cap_records,
+                       int64_t *d_counts, int64_t *d_status, void *d_ws, int64_t ws_bytes, pg_stream_t stream);
+
 /* ---- BGZF input: gzip members of at most 64 KiB, each a self-contained raw-DEFLATE stream -------
  * (the `bgzip` / `samtools faidx` format: gzip header with FLG = FEXTRA and a "BC" extra subfield of
  * SLEN 2 holding BSIZE = member size - 1; CRC-32 and ISIZE trailer).  A concatenation of BGZF files is

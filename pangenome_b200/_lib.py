@@ -15,6 +15,9 @@ PG_ERR_NOT_BGZF = -5
 PG_INF_ERRORS = {1: "bad header", 2: "truncated deflate data", 3: "invalid block type", 4: "stored block length check",
                  5: "invalid code lengths", 6: "invalid code", 7: "distance too far back", 8: "more output than ISIZE",
                  9: "length mismatch", 10: "CRC-32 mismatch"}
+# FASTQ input (include/pgdbg.h PG_FQ_*): the malformed-record kinds pg_fastq_scan_pack's d_status reports
+PG_FQ_ERRORS = {1: "header line does not start with '@'", 2: "separator line does not start with '+'",
+                3: "quality length differs from sequence length", 4: "truncated record (line count not a multiple of 4)"}
 PG_MCL_WARP_PRODUCTS, PG_MCL_SMEM_SLOTS = 64, 2048
 PG_MCL_STAT_CHAOS, PG_MCL_STAT_NNZ, PG_MCL_STAT_PRODUCTS, PG_MCL_STAT_MAXPROD, PG_MCL_STAT_LARGE, PG_MCL_STAT_WORDS = 0, 1, 2, 3, 4, 8
 
@@ -64,6 +67,8 @@ SIGNATURES = {
     "pg_pack_words": (c_i64, [c_i64]),
     "pg_fasta_workspace_bytes": (c_i64, [c_i64]),
     "pg_fasta_scan_pack": (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp]),
+    "pg_fastq_workspace_bytes": (c_i64, [c_i64, c_i64]),
+    "pg_fastq_scan_pack": (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_vp, c_vp, c_i64, c_vp]),
     "pg_table_bytes": (c_i64, [c_i64]),
     "pg_table_clear": (c_int, [PT, c_vp]),
     "pg_table_reset": (c_int, [PT, c_vp]),

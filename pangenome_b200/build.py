@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpgdbg.so")
-SOURCES = ["common.cu", "fasta_pack.cu", "dbg_table.cu", "path_graph.cu", "partition.cu", "region_build.cu", "multisplit.cu", "compact_build.cu", "host_io.cu", "microbench.cu", "mcl.cu", "bgzf_inflate.cu"]
+SOURCES = ["common.cu", "fasta_pack.cu", "dbg_table.cu", "path_graph.cu", "partition.cu", "region_build.cu", "multisplit.cu", "compact_build.cu", "host_io.cu", "microbench.cu", "mcl.cu", "bgzf_inflate.cu", "fastq_pack.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2"]
 

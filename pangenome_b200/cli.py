@@ -12,9 +12,11 @@ parser, so scripts stay portable): ``--min-edge-weight W``, ``--no-mcl-file``, `
 edge list (the default) or from Markov clustering on the GPU with inflation R (default 1.5, what the reference passes
 to ``mcl -I``; R > 1) in place of the reference's external ``mcl`` run.  An existing ``<xyz>.mcl`` still wins.
 
-Input: plain FASTA, or FASTA compressed by ``bgzip`` (BGZF: its members are inflated on the GPU) or by ``gzip``
+Input: plain FASTA or FASTQ, or either compressed by ``bgzip`` (BGZF: its members are inflated on the GPU) or by ``gzip``
 (inflated on the host).  Side files keep the name given with ``-i`` (``input.fa.gz_rdbg_weight.xyz``, ``input.fa.gz_db.npz``);
-``-r`` checkpoint offsets are positions in the decompressed stream.
+``-r`` checkpoint offsets are positions in the decompressed stream.  A FASTQ file (first byte '@'; four-line records)
+gives exactly what the FASTA of its header and sequence lines gives; quality lines are checked for length only.  A
+malformed FASTQ exits naming the byte offset of its first bad record.  ``-r`` takes FASTA only.
 
 Multi-GPU: ``torchrun --nproc-per-node N kmer_b200.py -i input.fasta -k 27`` - every rank packs its
 record-aligned byte range of the one input file, the dBG is hash-partitioned across the GPUs
@@ -118,6 +120,8 @@ def entry_point(argv, out=sys.stdout):
                          "GPU path; -r (dBG checkpoint) is")
     world, rank = _init_distributed()
     from . import stages
+    if args['-r'] and stages.seq_chk(qry) == "fastq":
+        raise SystemExit("pangenome_b200: -r (dBG checkpoint resume) reads FASTA only; %s is FASTQ" % qry)
     p = (lambda *a: print(*a, file=out)) if rank == 0 else (lambda *a: None)      # rank 0 owns stdout and the side files
     dbs, rdb = args['-d'], args['-D']
     if world > 1 and (dbs or rdb or args['-r']):

@@ -53,14 +53,19 @@ def to_device_bytes(data, device="cuda"):
 
 class PackedSeqs:
     """Result of K1 (pg_fasta_scan_pack): the 2-bit packed base stream plus the
-    record index.  Replaces what seqio_jit_ (kmer_numba.py:135-168) yields."""
+    record index.  Replaces what seqio_jit_ (kmer_numba.py:135-168) yields.
+    ``fmt="fastq"``: the same outputs from a FASTQ stream (pg_fastq_scan_pack), as the FASTA of its header and sequence
+    lines would give them; a malformed file raises FastqError when the record index is read."""
 
-    def __init__(self, d_fasta, cap_records=1 << 12, lazy=False):
+    def __init__(self, d_fasta, cap_records=1 << 12, lazy=False, fmt="fasta"):
         """``lazy``: enqueue K1 and return without reading the record index back; ``n_rec``,
         ``seq_off`` ... are fetched (one D2H, synchronising) the first time the host asks for them.
         The device-argument kernels (pg_kmer_partition_dev, ...) never need them on the host."""
         _require_cuda()
+        if fmt not in ("fasta", "fastq"):
+            raise PgError("PackedSeqs: fmt must be 'fasta' or 'fastq', got %r" % (fmt,))
         self.L = L = _lib.load()
+        self.fmt = fmt
         self.d_fasta = d_fasta
         nbytes = int(d_fasta.numel())
         dev = d_fasta.device
@@ -68,26 +73,37 @@ class PackedSeqs:
         words = int(L.pg_pack_words(nbytes))
         self.pk2 = torch.empty(words, dtype=torch.int32, device=dev)
         self.amb = torch.empty(words, dtype=torch.int32, device=dev)
-        self._ws_bytes = int(L.pg_fasta_workspace_bytes(nbytes))
-        self._ws = torch.empty(self._ws_bytes, dtype=torch.uint8, device=dev)
-        self.launches = 3
+        if fmt == "fasta":
+            self._ws_bytes = int(L.pg_fasta_workspace_bytes(nbytes))
+            self._ws = torch.empty(self._ws_bytes, dtype=torch.uint8, device=dev)
+        self.launches = 3 if fmt == "fasta" else 5
         self._host = None
         self._launch(cap_records)
         if not lazy:
             self._fetch()
 
     def _launch(self, cap_records):
-        # counts, seq_off and hdr_off share ONE device buffer so the record index comes back in one D2H
+        # counts, seq_off and hdr_off (and the FASTQ status) share ONE device buffer so the record index comes back in one D2H
         L, nbytes = self.L, self.nbytes
         self.cap_records = cap_records
-        idx = torch.empty(4 + (cap_records + 2) + (cap_records + 1), dtype=torch.int64, device=self.pk2.device)
+        fq = self.fmt == "fastq"
+        idx = torch.empty(4 + (cap_records + 2) + (cap_records + 1) + (2 if fq else 0), dtype=torch.int64, device=self.pk2.device)
         self._idx = idx
         self.d_counts = idx[:4]
         self.d_seq_off = idx[4:4 + cap_records + 2]
-        self.d_hdr_off = idx[4 + cap_records + 2:]
-        check(L.pg_fasta_scan_pack(_ptr(self.d_fasta) if nbytes else None, nbytes, _ptr(self.pk2), _ptr(self.amb),
-                                   nbytes, _ptr(self.d_hdr_off), _ptr(self.d_seq_off), cap_records,
-                                   _ptr(self.d_counts), _ptr(self._ws), self._ws_bytes, _stream()), "pg_fasta_scan_pack")
+        self.d_hdr_off = idx[4 + cap_records + 2:4 + cap_records + 2 + cap_records + 1]
+        src = _ptr(self.d_fasta) if nbytes else None
+        if not fq:
+            check(L.pg_fasta_scan_pack(src, nbytes, _ptr(self.pk2), _ptr(self.amb), nbytes, _ptr(self.d_hdr_off),
+                                       _ptr(self.d_seq_off), cap_records, _ptr(self.d_counts), _ptr(self._ws), self._ws_bytes,
+                                       _stream()), "pg_fasta_scan_pack")
+            return
+        self.d_status = idx[-2:]
+        self._ws_bytes = int(L.pg_fastq_workspace_bytes(nbytes, cap_records))
+        self._ws = torch.empty(self._ws_bytes, dtype=torch.uint8, device=self.pk2.device)
+        check(L.pg_fastq_scan_pack(src, nbytes, _ptr(self.pk2), _ptr(self.amb), nbytes, _ptr(self.d_hdr_off),
+                                   _ptr(self.d_seq_off), cap_records, _ptr(self.d_counts), _ptr(self.d_status), _ptr(self._ws),
+                                   self._ws_bytes, _stream()), "pg_fastq_scan_pack")
 
     def _fetch(self):
         if self._host is not None:
@@ -104,6 +120,10 @@ class PackedSeqs:
             if n_rec <= cap:
                 break
             self._launch(next_pow2(n_rec + 1))           # the index was truncated: pack again with room for it
+        if self.fmt == "fastq":
+            off, kind = (h[-2:] if h is not None else self.d_status.cpu().numpy()).tolist()
+            if off >= 0:
+                raise FastqError(off, kind)
         if h is not None:
             seq_off = h[4:4 + n_rec + 1].copy()
             hdr_off = h[4 + cap + 2:4 + cap + 2 + n_rec].copy()
@@ -142,6 +162,19 @@ class PackedSeqs:
         """The metric's unit: sum over record-strands of max(n-k+1, 1)."""
         lens = self.seq_lengths[:n_rec]
         return int(np.maximum(lens - k + 1, 1).sum()) * (2 if rc else 1)
+
+
+class FastqError(PgError):
+    """A malformed FASTQ stream: ``offset`` = byte offset (in the packed stream) of the first bad record's header line,
+    ``kind`` = include/pgdbg.h PG_FQ_* code."""
+
+    def __init__(self, offset, kind):
+        self.offset, self.kind = int(offset), int(kind)
+        super().__init__("malformed FASTQ: the record at byte %d: %s" % (self.offset, self.reason))
+
+    @property
+    def reason(self):
+        return _lib.PG_FQ_ERRORS.get(self.kind, "error %d" % self.kind)
 
 
 class _StatsFuture:

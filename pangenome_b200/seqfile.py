@@ -1,5 +1,5 @@
 """Reading the input sequence file.  The one place that knows about input formats: it looks at the first bytes and
-hands the rest of the package the DECOMPRESSED FASTA stream, on the device for K1 (``engine.PackedSeqs``) and on the
+hands the rest of the package the DECOMPRESSED FASTA or FASTQ stream (``detect`` tells which), on the device for K1 (``engine.PackedSeqs``) and on the
 host for what reads header text and byte offsets (``graph.record_ids``, the chunked build and its checkpoints).
 
 - plain FASTA: the file is mapped (np.memmap) and copied to the device as it is;
@@ -21,6 +21,25 @@ import numpy as np
 from . import _lib, shard
 
 GZIP_MAGIC = b"\x1f\x8b"
+
+
+def detect(first):
+    """Format of a decompressed stream from its first bytes (``head``): "fastq" when the first byte is '@', "fasta" when
+    it is '>' or a line starts with '>' (the reference's seq_chk, kmer_numba.py:873-886), then "fastq" when a line starts
+    with '@'; None otherwise.  A FASTQ file whose quality line starts with '>' is still FASTQ."""
+    first = bytes(first)
+    if first[:1] == b"@":
+        return "fastq"
+    if first[:1] == b">" or b"\n>" in first:
+        return "fasta"
+    if b"\n@" in first:
+        return "fastq"
+    return None
+
+
+def input_format(path):
+    """detect() of the first 40 bytes of the decompressed input."""
+    return detect(head(path, 40))
 
 
 def _map(path):
@@ -119,19 +138,20 @@ def _gunzip(buf):
 
 
 def read_rank_range(path, world, rank):
-    """This rank's record-aligned range of the decompressed input (shard.py's cut rule): (bytes, (begin, end),
+    """This rank's record-aligned range of the decompressed input (shard.py's cut rule for its format): (bytes, (begin, end),
     decompressed size).  BGZF: only the members around the range are inflated (shard.member_rank_range), on the GPU."""
     buf = _map(path)
     kind, idx = _kind(buf)
+    fmt = input_format(path)
     if kind == "plain":
-        return shard.plain_rank_range(path, world, rank)
+        return shard.plain_rank_range(path, world, rank, fmt)
     if kind == "gzip":
         raw = _gunzip(buf)
-        cuts = shard.cut_points(raw, world)
+        cuts = shard.cut_points(raw, world, fmt)
         return raw[cuts[rank]:cuts[rank + 1]], (cuts[rank], cuts[rank + 1]), len(raw)
     member_off, out_off = idx
     return shard.member_rank_range(out_off, world, rank,
-                                   lambda i0, i1: inflate_members(buf, member_off, out_off, i0, i1).cpu().numpy().tobytes())
+                                   lambda i0, i1: inflate_members(buf, member_off, out_off, i0, i1).cpu().numpy().tobytes(), fmt)
 
 
 def head(path, n=40):

@@ -40,15 +40,29 @@ def _dist_env():
 
 
 def seq_chk(qry):
-    """kmer_numba.py:873-886: peek 40 bytes, '>' anywhere at a line start -> fasta.  The bytes are those of the
-    decompressed stream when the file is gzip / BGZF compressed."""
+    """kmer_numba.py:873-886: peek 40 bytes, '>' anywhere at a line start -> fasta; but '@' as the first byte -> fastq
+    (seqfile.detect).  The bytes are those of the decompressed stream when the file is gzip / BGZF compressed."""
     from . import seqfile
-    s = seqfile.head(qry, 40)
-    if s[:1] == b">" or b"\n>" in s:
-        return "fasta"
-    if s[:1] == b"@" or b"\n@" in s:
-        return "fastq"
-    return None
+    return seqfile.input_format(qry)
+
+
+def _pack(qry, d_bytes, fmt, begin=0, world=1):
+    """PackedSeqs of the device bytes.  A malformed FASTQ exits naming the byte offset (in the decompressed input) of its
+    first bad record; ``begin`` = where this rank's range starts.  Under torchrun every rank learns whether any range was
+    malformed, so all of them stop before the first collective of the build."""
+    err = None
+    try:
+        packed = engine.PackedSeqs(d_bytes, fmt=fmt)
+    except engine.FastqError as e:
+        packed, err = None, (begin + e.offset, e.reason)
+    if world > 1 and fmt == "fastq":
+        import torch.distributed as dist
+        errs = [None] * world
+        dist.all_gather_object(errs, err)
+        err = min((e for e in errs if e is not None), default=None)
+    if err is not None:
+        raise SystemExit("pangenome_b200: %s: malformed FASTQ: the record at byte %d: %s" % (qry, err[0], err[1]))
+    return packed
 
 
 def seq2rdbg(qry, kmer=13, bits=5, Ns=1e6, chunk=2 ** 32, brkpt="./breakpoint", saved="dBG_disk", hashfunc=None,
@@ -58,31 +72,37 @@ def seq2rdbg(qry, kmer=13, bits=5, Ns=1e6, chunk=2 ** 32, brkpt="./breakpoint", 
     Chunk checkpoints as upstream (:1252-1266): whenever a call has consumed more than ``chunk`` bases
     (both strands counted) the table is written to ``<qry>_db_brkpt.npz`` together with the byte offset
     of the next header line; an existing ``brkpt`` file (``-r``) is loaded and the build resumes at its
-    offset.  Inputs below ``chunk`` with no ``brkpt`` file take the one-shot two-phase build."""
+    offset.  Inputs below ``chunk`` with no ``brkpt`` file take the one-shot two-phase build.
+
+    A FASTQ input gives what the FASTA of its header and sequence lines gives, and always takes the one-shot build:
+    the checkpoint loop and its offsets are those of the reference's FASTA reader, so resuming from ``brkpt`` exits."""
     if bits != 5:
         raise ValueError("only the reference's base-5 code (bits=5) is supported")
     kmer = min(max(1, int(kmer)), 27)
     world, rank = _dist_env()
-    d_bytes = None
+    d_bytes, fmt, begin = None, "fasta", 0
+    resume = bool(brkpt) and os.path.isfile(brkpt)
     if data is None:
-        if seq_chk(qry) != "fasta":
-            raise SystemExit("pangenome_b200: %s is not FASTA (the reference's fastq branch is broken upstream)" % qry)
+        fmt = seq_chk(qry)
+        if fmt not in ("fasta", "fastq"):
+            raise SystemExit("pangenome_b200: %s is neither FASTA nor FASTQ" % qry)
+        if fmt == "fastq" and resume:
+            raise SystemExit("pangenome_b200: -r (dBG checkpoint resume) reads FASTA only; %s is FASTQ" % qry)
         if world > 1:      # this rank's record-aligned byte range of the one file (SURVEY 8e)
             from . import shard
-            data, _, _ = shard.read_rank_range(qry, world, rank)
+            data, (begin, _), _ = shard.read_rank_range(qry, world, rank)
             data = np.frombuffer(data, dtype=np.uint8)
         else:
             data, d_bytes = _read(qry)
-    packed = engine.PackedSeqs(d_bytes if d_bytes is not None else engine.to_device_bytes(data))
+    packed = _pack(qry, d_bytes if d_bytes is not None else engine.to_device_bytes(data), fmt, begin, world)
     strands = 2 if rc else 1
-    resume = bool(brkpt) and os.path.isfile(brkpt)
     from . import builder
     if world > 1:
         if resume:
             raise SystemExit("pangenome_b200: -r (dBG checkpoint resume) runs on one GPU; launch without torchrun")
         table, n_rec, b = builder.build_table(packed, kmer, rc=bool(rc), Ns=Ns, world=world, rank=rank)
         return DbgHandle(table, packed, data, n_rec, world, rank, b)
-    if not resume and strands * int(packed.n_bases) <= chunk:
+    if fmt == "fastq" or (not resume and strands * int(packed.n_bases) <= chunk):
         # the streaming two-phase build (K2a partition + K3 region sweep): what bench.py times
         table, n_rec, b = builder.build_table(packed, kmer, rc=bool(rc), Ns=Ns)
         return DbgHandle(table, packed, data, n_rec, builder=b)
@@ -190,8 +210,9 @@ def load_dbg(qry, fn, kmer):
     """``-d`` / ``-D``: a table saved by the reference (or by ``dump``) + the packed input."""
     from . import npz
     kmer = min(max(1, int(kmer)), 27)
+    fmt = seq_chk(qry)
     data, d_bytes = _read(qry)
-    packed = engine.PackedSeqs(d_bytes)
+    packed = _pack(qry, d_bytes, "fastq" if fmt == "fastq" else "fasta")
     table = npz.load(fn, kmer, device=packed.pk2.device)
     return DbgHandle(table, packed, data, packed.n_rec)
 

@@ -144,6 +144,50 @@ def n_kmer_insertions(seq_lengths, k, rc=True):
     return tot * (2 if rc else 1)
 
 
+def reads(genomes_fasta, n_reads, length=150, n_rate=0.002, seed=7, batch=1 << 16):
+    """A seeded short-read set over the genomes of a FASTA image (e.g. ``pangenome()``): ``n_reads`` reads of ``length``
+    bases, genome and start uniform, half of them reverse-complemented, each base replaced by 'N' with probability
+    ``n_rate``; Illumina-like names ``SIM:1:FC:1:<tile>:<x>:<y> 1:N:0:<genome>`` and quality strings (Phred+33, falling
+    towards the 3' end, '#' on the Ns).  Returns the FASTQ bytes."""
+    rng = np.random.default_rng(seed)
+    genomes = [b"".join(rec.split(b"\n")[1:]) for rec in genomes_fasta.split(b">")[1:]]
+    genomes = [np.frombuffer(g, dtype=np.uint8) for g in genomes if len(g) >= length]
+    comp = np.arange(256, dtype=np.uint8)
+    comp[list(b"ACGT")] = list(b"TGCA")
+    decay = np.linspace(0, 12, length)
+    col = np.arange(length)
+    out = []
+    for r0 in range(0, n_reads, batch):
+        nb = min(batch, n_reads - r0)
+        g_idx = rng.integers(0, len(genomes), nb)
+        seqs = np.empty((nb, length), dtype=np.uint8)
+        for g, genome in enumerate(genomes):
+            m = np.nonzero(g_idx == g)[0]
+            starts = rng.integers(0, genome.size - length + 1, m.size)
+            seqs[m] = genome[starts[:, None] + col]
+        rev = rng.random(nb) < 0.5
+        seqs[rev] = comp[seqs[rev][:, ::-1]]
+        seqs[rng.random((nb, length)) < n_rate] = ord("N")
+        qual = (np.clip(rng.normal(38, 2, (nb, length)) - decay, 2, 41) + 33).astype(np.uint8)
+        qual[seqs == ord("N")] = ord("#")
+        xy = rng.integers(1000, 30000, (nb, 2))
+        for i in range(nb):
+            r = r0 + i
+            out.append(b"@SIM:1:FC:1:%d:%d:%d 1:N:0:%d\n%s\n+\n%s\n" % (1101 + r // 100000, xy[i, 0], xy[i, 1], g_idx[i],
+                                                                        seqs[i].tobytes(), qual[i].tobytes()))
+    return b"".join(out)
+
+
+def fastq_to_fasta(fq):
+    """fasta(F) of a valid four-line FASTQ image: each record's header with '>' for '@' (line ending kept), then its
+    sequence line as it is - the FASTA a FASTQ input is processed as.  Blank lines after the last record are dropped."""
+    lines = fq.split(b"\n")
+    if lines[-1] == b"":
+        lines.pop()
+    last = max((i for i, l in enumerate(lines) if l), default=-1)
+    return b"".join(b">" + lines[4 * r][1:] + b"\n" + lines[4 * r + 1] + b"\n" for r in range(last // 4 + 1))
+
+
 # the empty member every BGZF file ends with (SAM/BAM specification 4.1.2)
 BGZF_EOF = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
 
