@@ -540,6 +540,38 @@ int pg_host_write_mcl(const char *path, const uint64_t *code, const uint32_t *v5
 int64_t pg_host_oakht_capacity(int64_t n_entries);
 int pg_host_build_oakht(const uint64_t *keys, const uint16_t *vals, const uint8_t *cnts, int64_t n, int64_t cap,
                         uint64_t *okeys, uint16_t *ovals, uint8_t *ocnts);
+/* The same image on the GPU (npz_dump.cu).
+ * pg_oakht_place: device entries d_keys/d_vals/d_cnts[n] (distinct keys, e.g. pg_table_export's) ->
+ *   d_okeys/d_ovals/d_ocnts[cap] (cap = pg_host_oakht_capacity(n)).  Placement in rounds: in round s every
+ *   unplaced entry bids for its s-th probe slot of oakht.pointer() if no earlier round took it, the
+ *   smallest key wins; the sentinel key 2^64-1 takes its first probe slot before round 0.  The image
+ *   depends only on the set of entries (it is not the host's insertion-order arrangement); every key is
+ *   found by pointer(), empty slots hold key 0, value 0, count 0, live slots count >= 1.  d_ws: at least
+ *   pg_oakht_place_workspace_bytes(n).  Synchronises the stream every few rounds to read the number of
+ *   entries left; PG_ERR_CAPACITY when some are still unplaced after 4096 rounds.
+ * pg_deflate_chunks: raw DEFLATE of chunks [first_chunk, first_chunk + n_chunks) of one member whose bytes
+ *   are the HOST header hdr[hdr_len] (hdr_len <= PG_DEFLATE_HDR_MAX: the .npy header) followed by the
+ *   device array d_data[data_len], cut into chunks of chunk_bytes (<= 65535).  Chunk first_chunk + i goes
+ *   to d_staging + i * slot_bytes (slot_bytes >= pg_deflate_slot_bytes(chunk_bytes), a multiple of 16);
+ *   d_sizes[i] = its compressed size, d_crcs[i] = the CRC-32 of its input.  Chunks are independent and
+ *   byte-aligned; only the member's last chunk sets BFINAL, so the chunks in order form one raw-DEFLATE
+ *   stream.  One CTA per chunk (csrc/deflate.cuh, which the CPU test harness compiles too).
+ * pg_deflate_compact: after pg_deflate_chunks on the same slab: d_sizes[0, n_chunks) -> exclusive offsets,
+ *   d_sizes[n_chunks] = the slab's compressed bytes (d_sizes holds n_chunks + 1 entries); the slots are
+ *   copied to d_out at those offsets.  d_state[0]: in, the CRC-32 of the member's bytes before this slab
+ *   (0 for the first); out, including it.  d_state[1] = the slab's compressed bytes.  total_bytes =
+ *   hdr_len + data_len of the member. */
+#define PG_DEFLATE_HDR_MAX 256
+int pg_oakht_place(const uint64_t *d_keys, const uint16_t *d_vals, const uint8_t *d_cnts, int64_t n, int64_t cap,
+                   uint64_t *d_okeys, uint16_t *d_ovals, uint8_t *d_ocnts, void *d_ws, int64_t ws_bytes, pg_stream_t stream);
+int64_t pg_oakht_place_workspace_bytes(int64_t n);
+int64_t pg_deflate_slot_bytes(int64_t chunk_bytes);
+int pg_deflate_chunks(const uint8_t *hdr, int64_t hdr_len, const uint8_t *d_data, int64_t data_len, int64_t chunk_bytes,
+                      int64_t first_chunk, int64_t n_chunks, uint8_t *d_staging, int64_t slot_bytes, int64_t *d_sizes,
+                      uint32_t *d_crcs, pg_stream_t stream);
+int pg_deflate_compact(const uint8_t *d_staging, int64_t slot_bytes, int64_t *d_sizes, const uint32_t *d_crcs,
+                       int64_t first_chunk, int64_t n_chunks, int64_t chunk_bytes, int64_t total_bytes, uint8_t *d_out,
+                       int64_t *d_state, pg_stream_t stream);
 
 /* ---- measurement support (SURVEY.md 8d: "a micro-benchmark ceiling (random atomicCAS + atomicOr into a table of the
  * same byte size)") - not part of the hot path.  n_ops operations, each on one pseudo-random 16-byte slot; the regions

@@ -110,6 +110,11 @@ SIGNATURES = {
     "pg_bgzf_inflate": (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp]),
     "pg_host_oakht_capacity": (c_i64, [c_i64]),
     "pg_host_build_oakht": (c_int, [c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp]),
+    "pg_oakht_place": (c_int, [c_vp, c_vp, c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp]),
+    "pg_oakht_place_workspace_bytes": (c_i64, [c_i64]),
+    "pg_deflate_slot_bytes": (c_i64, [c_i64]),
+    "pg_deflate_chunks": (c_int, [ctypes.c_char_p, c_i64, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp]),
+    "pg_deflate_compact": (c_int, [c_vp, c_i64, c_vp, c_vp, c_i64, c_i64, c_i64, c_i64, c_vp, c_vp, c_vp]),
     "pg_path_workspace_bytes": (c_i64, [c_i64]),
     "pg_path_hits": (c_int, [PT, c_vp, c_vp, c_vp, c_i64, c_i64, c_i64, c_int, c_vp, c_vp, c_vp, c_vp, c_i64, c_vp, c_vp,
                              c_i64, c_vp]),

@@ -273,8 +273,9 @@ class DbgTable:
         v = out.cpu().numpy().view(np.uint64)
         return int(v[0]), int(v[1]), int(v[2])
 
-    def export(self, sort=True):
-        """(keys u64, vals u16, cnts u8) in the reference's convention."""
+    def export_device(self):
+        """The unsorted entries of ``export`` left on the device: (keys int64, vals int16, cnts uint8) tensors holding
+        the bits of u64 / u16 / u8."""
         _, n = self.count()
         dev = self.slots.device
         keys = torch.empty(max(n, 1), dtype=torch.int64, device=dev)
@@ -286,9 +287,14 @@ class DbgTable:
         got = int(d_n.item())
         if got != n:
             raise PgError("pg_table_export produced %d entries, pg_table_count said %d" % (got, n))
-        k = keys[:n].cpu().numpy().view(np.uint64)
-        v = vals[:n].cpu().numpy().view(np.uint16)
-        c = cnts[:n].cpu().numpy()
+        return keys[:n], vals[:n], cnts[:n]
+
+    def export(self, sort=True):
+        """(keys u64, vals u16, cnts u8) in the reference's convention."""
+        keys, vals, cnts = self.export_device()
+        k = keys.cpu().numpy().view(np.uint64)
+        v = vals.cpu().numpy().view(np.uint16)
+        c = cnts.cpu().numpy()
         if sort:
             o = np.argsort(k, kind="stable")
             k, v, c = k[o], v[o], c[o]

@@ -52,6 +52,102 @@ def gather_export(table, world, rank):
     return K[o], V[o], C[o]
 
 
+_PAIR_GROUPS = {}
+GATHER_PIECE = 64 << 20       # bytes one rank sends to rank 0 per broadcast
+
+
+def _pair_groups(world):
+    """The process groups {0, r}, r = 1 .. world - 1: a broadcast from r inside one reaches rank 0 alone, for NCCL and
+    for gloo on CUDA tensors alike (gloo has no point-to-point or gather for CUDA tensors).  Collective: every rank
+    creates every pair, in order, once per default group."""
+    key = (id(dist.group.WORLD), world)
+    if key not in _PAIR_GROUPS:
+        _PAIR_GROUPS[key] = [None] + [dist.new_group([0, q]) for q in range(1, world)]
+    return _PAIR_GROUPS[key]
+
+
+def gather_entries_rank0(table, world, rank, fits=None):
+    """The distributed dBG's entries on rank 0 only, moved as device tensors (sizes first, then each rank's bytes in
+    pieces of GATHER_PIECE): each rank drops its short-record sentinel and rank 0 adds one whose count is the sum over
+    ranks, clamped to 255 (the rule of gather_export).  ``fits(n)``: rank 0's choice, given the number of entries,
+    between device arrays (True) and host arrays received through a device bounce buffer (False).
+    Returns on rank 0 (on_device, keys, vals, cnts) - int64 / int16 / uint8 tensors, or u64 / u16 / u8 numpy arrays -
+    and None elsewhere."""
+    k, v, c = table.export_device()
+    dev = k.device
+    keep = k != -1
+    k, v, c = k[keep], v[keep], c[keep]
+    short = int(table.stats_host()[_lib.PG_STAT_SHORT])
+    mine = torch.tensor([k.numel(), short], dtype=torch.int64, device=dev)
+    sizes = [torch.zeros_like(mine) for _ in range(world)]
+    dist.all_gather(sizes, mine)
+    ns = [int(s[0]) for s in sizes]
+    tot_short = sum(int(s[1]) for s in sizes)
+    total = sum(ns) + (1 if tot_short > 0 else 0)
+    parts = [(k, 8), (v, 2), (c, 1)]
+    groups = _pair_groups(world)
+    if rank == 0:
+        on_dev = True if fits is None else bool(fits(total))
+        if on_dev:
+            out = [torch.empty(total, dtype=t.dtype, device=dev) for t, _ in parts]
+        else:
+            out = [torch.from_numpy(np.empty(total, dtype=d)) for d in (np.int64, np.int16, np.uint8)]
+        for o, (t, _) in zip(out, parts):
+            o[:ns[0]].copy_(t)
+        bounce = None if on_dev else torch.empty(GATHER_PIECE, dtype=torch.uint8, device=dev)
+    for r in range(1, world):
+        if rank not in (0, r):
+            continue
+        g = groups[r]
+        base = sum(ns[:r])
+        for i, (t, width) in enumerate(parts):
+            step = GATHER_PIECE // width
+            for a in range(0, ns[r], step):
+                m = min(step, ns[r] - a)
+                if rank == r:
+                    dist.broadcast(t[a:a + m].view(torch.uint8), src=r, group=g)
+                elif on_dev:
+                    dist.broadcast(out[i][base + a:base + a + m].view(torch.uint8), src=r, group=g)
+                else:
+                    buf = bounce[:m * width]
+                    dist.broadcast(buf, src=r, group=g)
+                    out[i][base + a:base + a + m].view(torch.uint8).copy_(buf.cpu())
+    if rank != 0:
+        return None
+    if tot_short > 0:
+        out[0][-1], out[1][-1], out[2][-1] = -1, 32, min(tot_short, 255)
+    if on_dev:
+        return True, out[0], out[1], out[2]
+    return False, out[0].numpy().view(np.uint64), out[1].numpy().view(np.uint16), out[2].numpy()
+
+
+def dump_rank0(table, world, rank, fn, budget=None):
+    """``<fn>.npz`` of the distributed dBG, written by rank 0 (other ranks return None after a barrier).  The entries
+    are gathered to rank 0 (gather_entries_rank0); rank 0 writes the image on the GPU when its free device memory (or
+    ``budget`` bytes) holds the gathered entries, the image and the encoder's slab pair, else on the host from the same
+    gather, and says so on stderr.  The file is the one the same entries give on one GPU."""
+    import sys
+    from . import npz
+    dev = table.slots.device
+
+    def fits(n):
+        room = budget if budget is not None else torch.cuda.mem_get_info(dev)[0]
+        return 11 * n + npz.device_bytes_needed(n) <= room
+
+    got = gather_entries_rank0(table, world, rank, fits)
+    out = None
+    if rank == 0:
+        on_dev, k, v, c = got
+        if on_dev:
+            out = npz.dump_device(k, v, c, fn)
+        else:
+            print("pangenome_b200: %d dBG entries do not fit rank 0's free device memory next to their image: "
+                  "writing %s.npz on the host" % (k.size, fn), file=sys.stderr)
+            out = npz.dump_entries(k, v, c, fn)
+    dist.barrier()
+    return out
+
+
 def gather_varlen(t, world):
     """Concatenation over ranks of 1-D tensors of different lengths (padded all_gather).
     Returns (concatenated tensor, per-rank lengths)."""

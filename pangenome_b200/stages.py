@@ -193,16 +193,14 @@ def _build_chunked(qry, raw, packed, kmer, Ns, chunk, brkpt, rc):
     return table
 
 
-def dump(kmer_dict, fn):
-    """kmer_numba.py dump (:243-261): ``<fn>.npz`` in the reference's oakht layout.  A hash-partitioned table is merged on
-    rank 0 first (every key lives on exactly one rank)."""
+def dump(kmer_dict, fn, budget=None):
+    """kmer_numba.py dump (:243-261): ``<fn>.npz`` in the reference's oakht layout.  A hash-partitioned table is gathered
+    to rank 0 first (every key lives on exactly one rank; the other ranks wait and return None).  ``budget``: the
+    device bytes rank 0 may use for the image (default: its free memory); beyond it rank 0 writes on the host."""
     from . import npz
     if kmer_dict.world > 1:
         from . import multigpu
-        merged = multigpu.gather_export(kmer_dict.table, kmer_dict.world, kmer_dict.rank)
-        if kmer_dict.rank != 0:
-            return None
-        return npz.dump_entries(*merged, fn)
+        return multigpu.dump_rank0(kmer_dict.table, kmer_dict.world, kmer_dict.rank, fn, budget=budget)
     return npz.dump(kmer_dict.table, fn)
 
 
